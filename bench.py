@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- cell-timesteps/sec of the fused energy-balance + melt kernel on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--mode f64_fast|f64|f32] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--mode f64_fast|f64|f32] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[3], SURVEY.md 8d cfg 4): a synthetic 4096 x 4096 glacierised raster
 (16 777 216 cells) PER GPU, hourly forcing, advanced in chunks of ``--chunk`` (default 128) timesteps.
@@ -20,6 +20,9 @@ One bench "step" = one launch of the fused kernel over one forcing chunk for eve
 
 ``--impl reference`` times that CPU port alone (the reference itself is a pure-Python package whose build
 backend is not installable offline, see DESIGN.md) and prints the line with "impl": "reference".
+
+``--dump-outputs DIR`` writes, after the timed launches, what the last of them handed its caller (``dump_outputs``).
+Cells and forcing are seeded, so two builds run with the same arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -41,6 +44,9 @@ UNIT = "cell-steps/s"
 GRID_CELLS = 4096 * 4096
 REGIONAL_CELLS = 100_000_000
 N_BASIN = 4096
+BMI_OUTPUTS = ("h_snow", "h_swe", "SM", "h_ice", "h_iwe", "IM", "M_total", "RH")
+DUMP_CELLS = 1 << 18          # cells sampled per state row: 2 MB each in float64
+DUMP_AGG_BYTES = 32 << 20     # basin aggregates: as many of the launch's last timesteps as fit
 
 
 def env_rank():
@@ -272,7 +278,8 @@ def run_reference_arm(args):
                       "timed as the slowest worker's compute time (pool start-up and pickling excluded)"}
     if reference_available():
         inst, steps_ref = args.ref_instances_per_core, 288
-        runs = [reference_throughput(cores, inst, steps_ref) for _ in range(max(1, min(args.steps, 3)))]
+        # --warmup untimed runs, then exactly --steps timed ones (--ref-instances-per-core bounds the cost of each)
+        runs = [reference_throughput(cores, inst, steps_ref) for _ in range(args.warmup + args.steps)][args.warmup:]
         value = sum(r[0] for r in runs) / len(runs)
         ms = 1e3 * sum(r[1] for r in runs) / len(runs)
         base = {"value": value, "unit": UNIT, "cores": cores, "kind": "reference",
@@ -359,6 +366,35 @@ def time_launches(eng, forcing, Tc, zero_agg, reduce_agg, steps, world, dev):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     return sum(a.elapsed_time(b) for a, b in evs) / len(evs), float(t.item())
+
+
+def dump_outputs(out_dir, eng, agg) -> None:
+    """Write what the last timed launch handed its caller to ``out_dir/<name>.npy``: the BMI output rows of the state
+    (``BMI_OUTPUTS``, engine dtype, ``[cells]``) and the launch's per-basin aggregates (float64 ``[timesteps, n_basin]``,
+    one file per ``sharding.AGG_NAMES`` entry, prefixed ``basin_``).
+
+    A row longer than ``DUMP_CELLS`` is cut to a fixed sample of that many cells (seed 0, ascending cell order), the
+    aggregates to the last timesteps that fit in ``DUMP_AGG_BYTES``: at most 48 MB in all, the same cells and
+    timesteps on every run with the same arguments.  With several ranks this is rank 0's shard of cells."""
+    import numpy as np
+    import torch
+
+    from topoflow_glacier_b200.sharding import AGG_NAMES
+
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    torch.cuda.synchronize()
+    cells = None
+    if eng.N > DUMP_CELLS:
+        pick = np.sort(np.random.default_rng(0).choice(eng.N, DUMP_CELLS, replace=False))
+        cells = torch.as_tensor(pick, device=eng.device)
+    for name in BMI_OUTPUTS:
+        row = eng.row(name)
+        np.save(out / f"{name}.npy", (row if cells is None else row[cells]).cpu().numpy())
+    n_t = max(1, min(agg.buffer.shape[0], DUMP_AGG_BYTES // (agg.buffer[0].numel() * 8)))
+    tail = agg.buffer[-n_t:].cpu().numpy()
+    for j, name in enumerate(AGG_NAMES):
+        np.save(out / f"basin_{name}.npy", np.ascontiguousarray(tail[..., j]))
 
 
 def run_gpu_arm(args):
@@ -480,6 +516,8 @@ def run_gpu_arm(args):
     t0 = time.perf_counter()
     (kern_ms, dev_ms), clocks = clocked(lambda: time_launches(eng, forcing, Tc, zero_agg, reduce_agg, args.steps, world, dev))
     wall = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:   # before the legs below advance the same engine further
+        dump_outputs(args.dump_outputs, eng, agg)
     cell_steps = n_cells * Tc  # this rank's launch
     value = total_cells * Tc * args.steps / (dev_ms * 1e-3)
 
@@ -515,7 +553,7 @@ def run_gpu_arm(args):
                 else torch.empty(Te, 6, n_cells, dtype=raw_dtype).pin_memory())
     raw_host.copy_(raw_dev)
     del raw_dev, raw_f, blk
-    out_names = ("h_snow", "h_swe", "SM", "h_ice", "h_iwe", "IM", "M_total", "RH")
+    out_names = BMI_OUTPUTS
     out_dtype = torch.float32 if args.e2e_out == "float32" else eng.dtype
     out_host = [torch.empty(len(out_names), n_cells, dtype=out_dtype).pin_memory() for _ in range(2)]
     drain = torch.cuda.Stream(device=dev)
@@ -791,7 +829,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-coherent", action="store_true")
     ap.add_argument("--no-shared", action="store_true", help="skip the catchment-forcing end-to-end leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed launches, write the outputs of the last one to DIR/<name>.npy (GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm; --impl reference has none")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     regional = args.workload == "regional"

@@ -293,22 +293,6 @@ def test_hydrofabric_topology_and_basin_ids(tmp_path):
         read_hydrofabric(tmp_path / "missing.gpkg")
 
 
-@pytest.mark.skipif(not Path("/root/reference/data/12082500.gpkg").exists(), reason="upstream checkout not present")
-def test_hydrofabric_shipped_gpkg_matches_configs():
-    """Build container only: the shipped GeoPackage gives the `da` values the yaml files carry."""
-    import yaml
-
-    from topoflow_glacier_b200.hydrofabric import read_hydrofabric
-
-    h = read_hydrofabric("/root/reference/data/12082500.gpkg")
-    assert len(h.divide_id) == 43 and abs(h.areasqkm.sum() - 361.0242) < 1e-3
-    for name in ("cat-3062784", "cat-3062920", "cat-3062924", "cat-3062927"):
-        cfg = yaml.safe_load(open(f"/root/reference/config/{name}.yaml"))
-        assert h.area_of([name])[0] == cfg["da"]
-    b, names = h.basin_ids(h.divide_id)
-    assert set(b) == {0} and len(names) == 1
-
-
 def test_pinned_block_needs_the_cuda_library():
     """forcing.pinned_block allocates through the C ABI (cudaHostAlloc): without a GPU it fails loudly instead of handing
     out pageable memory; tfg_host_is_pinned answers 0 for ordinary host memory."""
