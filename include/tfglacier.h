@@ -168,6 +168,31 @@ TFG_API int tfg_bind_mass_residual(tfg_ctx* ctx, void* lo);
  * reference's one-CSV-per-catchment drivers do (examples/run_topoflow_glacier.py:30-49), without replicating it per
  * cell on the host or over PCIe.  NULL restores the default, one column per cell.  Call after tfg_bind_static.    */
 TFG_API int tfg_bind_forcing_map(tfg_ctx* ctx, const int32_t* forcing_col, int64_t n_cols);
+/* Optional per-cell surface parameters: each field is a dev float64 array of length n_cells (in every mode), or NULL
+ * for "use the context constant" of the same name.  Where each one enters the reference:
+ *   dust_atten     atmospheric transmissivity and scattering of clear-sky radiation (solar_funcs.py:894-953)
+ *   canopy_factor  Brutsaert air emissivity, em_air = (1 - F) 1.72 (e/T)^(1/7) (1 + 0.22 C^2) + F (:1167-1180)
+ *   cloud_factor   the same expression, through C
+ *   z0_air         log-law aerodynamic conductance, ln((z - h_snow) / z0_air) (:670)
+ *   em_surf        outgoing longwave, em_surf sigma T_surf^4 + (1 - em_surf) LW_in (:1236-1246)
+ * Ranges of the configuration schema: dust_atten [0, 0.2], canopy_factor [0, 1], cloud_factor [0, 1],
+ * z0_air [1e-4, 0.1], em_surf [0.9, 1].                                                                      */
+typedef struct tfg_cell_params {
+  const double* dust_atten;
+  const double* canopy_factor;
+  const double* cloud_factor;
+  const double* z0_air;
+  const double* em_surf;
+} tfg_cell_params;
+
+/* Bind (p != NULL) or unbind (p == NULL) per-cell surface parameters; call after tfg_bind_static and tfg_set_constants,
+ * and again after either changes.  May be called between launches (a calibration loop).  The library derives the
+ * factors the kernels read (the per-cell counterparts of what tfg_set_constants derives from the constants) into a
+ * scratch it owns, on `stream`, and checks every value on the device: a non-finite value or one outside the ranges
+ * above is an error, after which no parameters are bound.  The call waits for that check; the caller's arrays are not
+ * read again afterwards.  A cell whose parameters equal the constants gives the bits of an unbound run.          */
+TFG_API int tfg_bind_cell_params(tfg_ctx* ctx, const tfg_cell_params* p, void* stream);
+
 /* host tables for steps [0, n_steps): rows[n_steps], gmt_offset_hours[n_steps][n_tz]; copied by the library
  * (each launch carries its <= 128 rows in the kernel parameter block); replaces solar.gmt_offset_hours,
  * solar_funcs.py:1616-1637, evaluated on the host                                                 */

@@ -36,6 +36,13 @@ class Constants(C.Structure):
         ("satterlund", C.c_int32), ("ring_slots", C.c_int32)]
 
 
+CELL_PARAM_FIELDS = ("dust_atten", "canopy_factor", "cloud_factor", "z0_air", "em_surf")
+
+
+class CellParams(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in CELL_PARAM_FIELDS]
+
+
 class TimeRow(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("clock_hour", "TE", "sin_decl", "cos_decl", "tan_decl", "isc_e0",
                                               "cos_hour", "sin_hour")]
@@ -74,6 +81,7 @@ PROTOTYPES = {
     "tfg_bind_static": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(Statics)]),
     "tfg_bind_state": (C.c_int, [C.c_void_p, C.POINTER(State)]),
     "tfg_bind_forcing_map": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64]),
+    "tfg_bind_cell_params": (C.c_int, [C.c_void_p, C.POINTER(CellParams), C.c_void_p]),
     "tfg_bind_window_carry": (C.c_int, [C.c_void_p, C.c_void_p]),
     "tfg_bind_mass_residual": (C.c_int, [C.c_void_p, C.c_void_p]),
     "tfg_bind_time": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),

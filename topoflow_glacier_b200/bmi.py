@@ -26,7 +26,7 @@ import torch
 import yaml
 
 from . import _lib
-from .config import TopoflowGlacierConfig
+from .config import CELL_PARAM_KEYS, KERNEL_CONSTANTS, TopoflowGlacierConfig
 from .engine import INPUT_ROWS, MeltEngine
 from .logger import configure_logging, logger
 from .statics import CELL_KEYS
@@ -37,7 +37,7 @@ try:  # the reference derives from bmipy.Bmi; keep that when the package is pres
 except Exception:  # noqa: BLE001
     _BmiBase = object
 
-__all__ = ["BmiTopoflowGlacier"]
+__all__ = ["BmiTopoflowGlacier", "ensemble_cell_params"]
 
 # (BMI name, unit, internal name) -- names and unit strings as in the reference, :18-57
 _INPUTS = (
@@ -62,6 +62,22 @@ _OUTPUTS = (
 INTERNAL_NAME_CROSSWALK = {b: i for b, _, i in _INPUTS + _OUTPUTS}
 EXTERNAL_NAME_CROSSWALK = {v: k for k, v in INTERNAL_NAME_CROSSWALK.items()}
 _OUT_INTERNAL = tuple(i for _, _, i in _OUTPUTS)
+
+
+def ensemble_cell_params(cfgs) -> dict:
+    """Per-member values of ``config.CELL_PARAM_KEYS`` (float64 ``[len(cfgs)]`` arrays) of an ensemble of validated configs.
+
+    Every other setting the kernels read is one value per model: members that differ in ``dt``, ``start_time``,
+    ``SATTERLUND`` or another ``KERNEL_CONSTANTS`` key are refused with a ``ValueError`` naming the key."""
+    head = cfgs[0]
+    for c in cfgs[1:]:
+        if (c.dt, str(c.start_time)) != (head.dt, str(head.start_time)):
+            raise ValueError("all ensemble members must share dt and start_time")
+        for k in ("SATTERLUND",) + tuple(k for k in KERNEL_CONSTANTS if k not in CELL_PARAM_KEYS):
+            if getattr(c, k) != getattr(head, k):
+                raise ValueError(f"all ensemble members must share {k} (only {', '.join(CELL_PARAM_KEYS)} may differ "
+                                 f"per member): {getattr(head, k)!r} != {getattr(c, k)!r}")
+    return {k: np.array([getattr(c, k) for c in cfgs], dtype=np.float64) for k in CELL_PARAM_KEYS}
 
 
 class BmiTopoflowGlacier(_BmiBase):
@@ -93,7 +109,8 @@ class BmiTopoflowGlacier(_BmiBase):
 
         ``engine_kw`` reaches ``MeltEngine``: e.g. ``mode="f64_fast"``, ``basin_id=..., n_basin=...`` or
         ``forcing_index=..., n_forcing_cols=M`` (members that share a forcing series: the input variables then hold
-        ``M`` values, one per series)."""
+        ``M`` values, one per series).  Each member keeps its own ``dust_atten, canopy_factor, cloud_factor, z0_air,
+        em_surf``; members that differ in any other physical constant are refused (``ensemble_cell_params``)."""
         cfgs = []
         for c in configs:
             if isinstance(c, (str, Path)):
@@ -108,7 +125,8 @@ class BmiTopoflowGlacier(_BmiBase):
 
         ``base_config`` (path, dict or validated object) supplies ``dt``, the time window and the physical constants;
         ``cells`` maps the per-catchment yaml keys (``statics.CELL_KEYS``: ``da, slope, aspect, lon, lat, elev,
-        h0_snow, h0_ice, h0_swe, h0_iwe, T_rain_snow``) to float64 ``[N]`` arrays.  ``zones`` / ``tz_idx`` as for
+        h0_snow, h0_ice, h0_swe, h0_iwe, T_rain_snow``) to float64 ``[N]`` arrays, and may also give per-cell values
+        of ``config.CELL_PARAM_KEYS`` (``dust_atten`` ... ``em_surf``; the others come from ``base_config``).  ``zones`` / ``tz_idx`` as for
         ``MeltEngine``; ``engine_kw`` reaches it too (``mode``, ``basin_id``, ``n_basin``, ``forcing_index`` ...).
         With ``shard=True`` under an initialised ``torch.distributed`` group every rank keeps only its own
         128-aligned block of the cells (``sharding.shard_bounds``) -- see ``ShardedMeltEngine``."""
@@ -117,7 +135,11 @@ class BmiTopoflowGlacier(_BmiBase):
             with open(c) as f:
                 c = yaml.safe_load(f)
         self.cfg = c if isinstance(c, TopoflowGlacierConfig) else TopoflowGlacierConfig.model_validate(c)
+        par = {k: np.atleast_1d(np.asarray(cells[k], dtype=np.float64)) for k in CELL_PARAM_KEYS if k in cells}
         cells = {k: np.atleast_1d(np.asarray(cells[k], dtype=np.float64)) for k in CELL_KEYS}
+        if par:
+            n = cells["lat"].size
+            engine_kw.setdefault("cell_params", {k: np.broadcast_to(v, (n,)) for k, v in par.items()})
         if zones is None:
             h = self.cfg
             zones = [h.utc_offset_hours if h.utc_offset_hours is not None else
@@ -126,9 +148,7 @@ class BmiTopoflowGlacier(_BmiBase):
 
     def _build(self, cfgs, **engine_kw) -> None:
         head = cfgs[0]
-        for c in cfgs[1:]:
-            if (c.dt, str(c.start_time)) != (head.dt, str(head.start_time)):
-                raise ValueError("all ensemble members must share dt and start_time")
+        engine_kw.setdefault("cell_params", ensemble_cell_params(cfgs))
         cells = {k: np.array([getattr(c, k) for c in cfgs], dtype=np.float64) for k in CELL_KEYS}
         zones, tz_idx = [], np.zeros(len(cfgs), dtype=np.uint8)
         for i, c in enumerate(cfgs):

@@ -16,7 +16,8 @@ from typing import Any, Optional
 
 from pydantic import ConfigDict, Field, create_model, field_validator
 
-__all__ = ["TopoflowGlacierConfig", "KERNEL_CONSTANTS", "default_constants"]
+__all__ = ["TopoflowGlacierConfig", "KERNEL_CONSTANTS", "CELL_PARAM_KEYS", "CELL_PARAM_RANGES", "check_cell_params",
+           "default_constants"]
 
 _REQ = ...  # pydantic's "required" marker
 
@@ -89,6 +90,26 @@ _TABLE: dict[str, tuple[type, Any, dict, str]] = {
 KERNEL_CONSTANTS = ("T0", "h_active_layer", "rho_air", "rho_snow", "rho_ice", "rho_H2O", "Cp_air", "Cp_snow",
                     "Cp_ice", "g", "Lf", "Lv", "eps", "kappa", "latent_heat_constant", "sigma", "sea_level_p0",
                     "uni_gas_const", "M_mass_air", "z0_air", "em_surf", "dust_atten", "canopy_factor", "cloud_factor")
+
+
+# per-catchment tunables that may also be given per cell (MeltEngine(cell_params=...), tfg_bind_cell_params)
+CELL_PARAM_KEYS = ("dust_atten", "canopy_factor", "cloud_factor", "z0_air", "em_surf")
+CELL_PARAM_RANGES = {k: (_TABLE[k][2]["ge"], _TABLE[k][2]["le"]) for k in CELL_PARAM_KEYS}
+
+
+def check_cell_params(params) -> dict:
+    """Validate per-cell parameter arrays (NumPy arrays or torch tensors, any device) against the schema's ranges.
+
+    Returns ``params`` as a plain dict; raises ``ValueError`` naming the first unknown key, or the first key holding a
+    value that is not finite or outside its range."""
+    params = dict(params)
+    for k, v in params.items():
+        if k not in CELL_PARAM_RANGES:
+            raise ValueError(f"{k!r} is not a per-cell parameter (one of {', '.join(CELL_PARAM_KEYS)})")
+        lo, hi = CELL_PARAM_RANGES[k]
+        if not bool(((v >= lo) & (v <= hi)).all()):   # NaN and +-inf compare false
+            raise ValueError(f"{k}: every value must be finite and within [{lo}, {hi}]")
+    return params
 
 
 def _coerce_time(cls, v):  # noqa: ANN001

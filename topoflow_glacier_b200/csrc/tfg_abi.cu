@@ -54,9 +54,51 @@ struct tfg_ctx {
   double* col_terms = nullptr;           // [<= kMaxLaunchSteps][n_cols][16] scratch of the column-term pass (owned)
   size_t col_terms_bytes = 0;
   int64_t col_term_launches = 0;         // launches that went through the column-term pass (tfg_column_term_launches)
+  void* cell_par = nullptr;              // [tfg::kPCount][n_cells] per-cell surface factors, context element type (owned)
+  size_t cell_par_bytes = 0;
+  int* cell_par_bad = nullptr;           // device flags of tfg_bind_cell_params' range check (owned)
+  bool have_cell_par = false;            // tfg_bind_cell_params: the scratch holds this context's factors
 };
 
 namespace {
+
+// Single-rounding operations on the host and on the device alike (the device compiler would otherwise contract
+// a*b + c into one FMA, and a per-cell factor would then differ from the constant the host derived).
+__host__ __device__ inline double mul_rn(double a, double b) {
+#ifdef __CUDA_ARCH__
+  return __dmul_rn(a, b);
+#else
+  return a * b;
+#endif
+}
+__host__ __device__ inline double add_rn(double a, double b) {
+#ifdef __CUDA_ARCH__
+  return __dadd_rn(a, b);
+#else
+  return a + b;
+#endif
+}
+__host__ __device__ inline double div_rn(double a, double b) {
+#ifdef __CUDA_ARCH__
+  return __ddiv_rn(a, b);
+#else
+  return a / b;
+#endif
+}
+
+// The factors the five surface parameters enter the kernels through, in the rows of tfg::kP*.  derive() forms them from
+// the context constants, cell_params_kernel from per-cell arrays: one statement of them keeps the two bit-identical.
+__host__ __device__ inline void surface_factors(double dust, double canopy, double cloud, double z0, double em_surf,
+                                                double sigma, double out[tfg::kPCount]) {
+  out[tfg::kPDust] = dust;
+  out[tfg::kPEmisA] = mul_rn(add_rn(1.0, -canopy), 1.72);                 // (1 - F) * 1.72 (:1179)
+  out[tfg::kPEmisB] = add_rn(1.0, mul_rn(0.22, mul_rn(cloud, cloud)));   // 1 + 0.22 * C**2 (:1180)
+  out[tfg::kPCanopy] = canopy;
+  out[tfg::kPEsSigma] = mul_rn(em_surf, sigma);                          // em_surf * sigma (:1236)
+  out[tfg::kPOneMEs] = add_rn(1.0, -em_surf);                            // 1 - em_surf (:1246)
+  out[tfg::kPZ0] = z0;
+  out[tfg::kPInvZ0] = div_rn(1.0, z0);
+}
 
 template <class raw>
 tfg::Consts<raw> derive(const tfg_constants& c) {
@@ -80,19 +122,21 @@ tfg::Consts<raw> derive(const tfg_constants& c) {
   k.wi_ratio = c.rho_H2O / c.rho_ice;
   k.rho_cp_snow = c.rho_snow * c.Cp_snow;
   k.rho_lf = c.rho_H2O * c.Lf;
-  k.dust = c.dust_atten;
-  k.emis_a = (1.0 - c.canopy_factor) * 1.72;
-  k.emis_b = 1.0 + (0.22 * (c.cloud_factor * c.cloud_factor));
-  k.canopy = c.canopy_factor;
+  double sf[tfg::kPCount];
+  surface_factors(c.dust_atten, c.canopy_factor, c.cloud_factor, c.z0_air, c.em_surf, c.sigma, sf);
+  k.dust = sf[tfg::kPDust];
+  k.emis_a = sf[tfg::kPEmisA];
+  k.emis_b = sf[tfg::kPEmisB];
+  k.canopy = sf[tfg::kPCanopy];
   k.sigma = c.sigma;
-  k.es_sigma = c.em_surf * c.sigma;
-  k.one_m_es = 1.0 - c.em_surf;
+  k.es_sigma = sf[tfg::kPEsSigma];
+  k.one_m_es = sf[tfg::kPOneMEs];
   k.one_seventh = 1.0 / 7.0;
   const double pi = 3.141592653589793;
   k.omega = (360.0 / 24.0) * (pi / 180.0);
   k.rad2deg = 180.0 / pi;
   k.deg2rad = pi / 180.0;
-  k.inv_z0 = 1.0 / c.z0_air;
+  k.inv_z0 = sf[tfg::kPInvZ0];
   k.inv_dt = 1.0 / c.dt_hours;
   k.inv_rho_lf = 1.0 / k.rho_lf;
   k.inv_rstar = 1.0 / c.uni_gas_const;
@@ -159,7 +203,33 @@ tfg::RunParams<raw> make_params(const tfg_ctx* x, const void* forcing, int64_t s
     p.agg_up[q] = ldexp(1.0, 40 - ((int)((x->exact_agg >> (8 * q)) & 0xff) - 128));
   p.n_basin = n_basin;
   p.k = derive<raw>(x->c);
+  p.cell_par = x->have_cell_par ? static_cast<const raw*>(x->cell_par) : nullptr;
   return p;
+}
+
+// ---- per-cell surface parameters (tfg_bind_cell_params) -----------------------------------------------------------
+// Ranges of the configuration schema (topoflow_glacier_b200/config.py); bit i of *bad = parameter i out of range.
+__global__ void cell_params_kernel(const tfg_cell_params in, const tfg_constants c, void* out, bool f32, int64_t N, int* bad) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= N) return;
+  const double* src[5] = {in.dust_atten, in.canopy_factor, in.cloud_factor, in.z0_air, in.em_surf};
+  const double dflt[5] = {c.dust_atten, c.canopy_factor, c.cloud_factor, c.z0_air, c.em_surf};
+  const double lo[5] = {0.0, 0.0, 0.0, 1e-4, 0.9}, hi[5] = {0.2, 1.0, 1.0, 0.1, 1.0};
+  double v[5];
+  int flags = 0;
+#pragma unroll
+  for (int j = 0; j < 5; ++j) {
+    v[j] = src[j] ? src[j][i] : dflt[j];
+    if (src[j] && !(v[j] >= lo[j] && v[j] <= hi[j])) flags |= 1 << j;   // NaN and +-inf fail too
+  }
+  if (flags) atomicOr(bad, flags);
+  double f[tfg::kPCount];
+  surface_factors(v[0], v[1], v[2], v[3], v[4], c.sigma, f);
+#pragma unroll
+  for (int r = 0; r < tfg::kPCount; ++r) {
+    if (f32) static_cast<float*>(out)[r * N + i] = (float)f[r];
+    else static_cast<double*>(out)[r * N + i] = f[r];
+  }
 }
 
 // ---- K2: raw met columns -> live forcings (examples/run_topoflow_glacier.py:40-73) -------------------
@@ -314,6 +384,8 @@ void tfg_destroy(tfg_ctx* x) {
   if (!x) return;
   cudaSetDevice(x->device);
   if (x->col_terms) cudaFree(x->col_terms);
+  if (x->cell_par) cudaFree(x->cell_par);
+  if (x->cell_par_bad) cudaFree(x->cell_par_bad);
   delete x;
 }
 
@@ -335,6 +407,7 @@ int tfg_set_constants(tfg_ctx* x, const tfg_constants* c) {
   if (c->ring_slots < 1 || c->ring_slots > TFG_RING_SLOTS_MAX) return fail("tfg_set_constants: bad ring_slots");
   x->c = *c;
   x->have_consts = true;
+  x->have_cell_par = false;  // the factors of unnamed parameters came from the old constants: bind again
   return 0;
 }
 
@@ -349,6 +422,45 @@ int tfg_bind_static(tfg_ctx* x, int64_t n_cells, const tfg_statics* s) {
   x->s = *s;
   x->n_cells = n_cells;
   x->have_static = true;
+  x->have_cell_par = false;  // sized for the old cell count: bind again
+  return 0;
+}
+
+int tfg_bind_cell_params(tfg_ctx* x, const tfg_cell_params* p, void* stream) {
+  if (!x) return fail("tfg_bind_cell_params: NULL context");
+  x->have_cell_par = false;
+  if (!p) return 0;
+#if defined(TFG_LEAN_W2) || TFG_WS || TFG_PIPELINE || TFG_SPLIT_STEP
+  return fail("tfg_bind_cell_params: this build runs an experimental kernel variant, which has no per-cell parameters");
+#endif
+  if (!x->have_static || !x->have_consts) return fail("tfg_bind_cell_params: call after tfg_set_constants and tfg_bind_static");
+  TFG_CUDA(cudaSetDevice(x->device));
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const size_t need = (size_t)tfg::kPCount * (size_t)x->n_cells * tfg_elem_size(x);
+  if (x->cell_par_bytes < need) {
+    if (x->cell_par) TFG_CUDA(cudaFree(x->cell_par));
+    x->cell_par = nullptr;
+    x->cell_par_bytes = 0;
+    TFG_CUDA(cudaMalloc(&x->cell_par, need));
+    x->cell_par_bytes = need;
+  }
+  if (!x->cell_par_bad) TFG_CUDA(cudaMalloc(&x->cell_par_bad, sizeof(int)));
+  TFG_CUDA(cudaMemsetAsync(x->cell_par_bad, 0, sizeof(int), s));
+  cell_params_kernel<<<(unsigned)((x->n_cells + 255) / 256), 256, 0, s>>>(*p, x->c, x->cell_par, x->mode == TFG_F32,
+                                                                         x->n_cells, x->cell_par_bad);
+  TFG_CUDA(cudaGetLastError());
+  int bad = 0;
+  TFG_CUDA(cudaMemcpyAsync(&bad, x->cell_par_bad, sizeof(int), cudaMemcpyDeviceToHost, s));
+  TFG_CUDA(cudaStreamSynchronize(s));
+  if (bad) {
+    static const char* names[5] = {"dust_atten [0, 0.2]", "canopy_factor [0, 1]", "cloud_factor [0, 1]", "z0_air [1e-4, 0.1]",
+                                   "em_surf [0.9, 1]"};
+    std::string m = "tfg_bind_cell_params: values not finite or outside their range:";
+    for (int j = 0; j < 5; ++j)
+      if (bad & (1 << j)) { m += " "; m += names[j]; }
+    return fail(m.c_str());
+  }
+  x->have_cell_par = true;
   return 0;
 }
 
@@ -444,8 +556,9 @@ int tfg_run(tfg_ctx* x, const void* forcing, int64_t step0, int32_t n_steps, voi
           else (void)cudaGetLastError();
         }
         if (x->col_terms_bytes >= need) {
-          e = strict ? tfg::launch_column_terms_strict(static_cast<const double*>(f), x->col_terms, nt, x->n_cols, p.k, s)
-                     : tfg::launch_column_terms_fast(static_cast<const double*>(f), x->col_terms, nt, x->n_cols, p.k, s);
+          const bool par = p.cell_par != nullptr;
+          e = strict ? tfg::launch_column_terms_strict(static_cast<const double*>(f), x->col_terms, nt, x->n_cols, p.k, par, s)
+                     : tfg::launch_column_terms_fast(static_cast<const double*>(f), x->col_terms, nt, x->n_cols, p.k, par, s);
           p.col_terms = x->col_terms;
           ++x->col_term_launches;
         }

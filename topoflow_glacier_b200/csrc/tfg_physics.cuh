@@ -124,17 +124,29 @@ enum { kSaElev, kSSinLat, kSCosLat, kSNegTanLat, kSSinEq, kSCosEq, kSNegTanEq, k
        kSCB, kSSB, kSCB2, kSSB2, kSVolP, kSVolPR, kSVolPS, kSVolSM, kSVolIM, kSPmax,
        kSaElevR,   // fast float64 only: a_elev / R*, formed once per launch instead of once per step
        kSCount };
+// Per-cell surface factors (tfg_bind_cell_params): the rows of the library's [kPCount][n_cells] scratch and, in kernels
+// instantiated with per-cell parameters, shared-memory columns kSCount + i.  Each replaces the Consts field of the
+// same meaning; the strict step divides by z0_air, the fast steps multiply by its reciprocal (the fast float64 kernel
+// needs both: its fallback for insane forcings and SATTERLUND is the strict step).
+enum { kPDust, kPEmisA, kPEmisB, kPCanopy, kPEsSigma, kPOneMEs, kPZ0, kPInvZ0, kPCount };
 
 template <class raw>
 struct RegCell {
+  static constexpr bool kPar = false;
   raw v[kSCount];
   __device__ __forceinline__ raw get(int i) const { return v[i]; }
   __device__ __forceinline__ void set(int i, raw x) { v[i] = x; }
+  __device__ __forceinline__ raw par(int, raw k) const { return k; }
 };
 
-template <class raw, int BLOCK>
+template <class raw, int BLOCK, bool PAR = false>
 struct SmemCell {
+  static constexpr bool kPar = PAR;   // per-cell surface factors in columns kSCount + kP*
   unsigned base;  // shared-window address of this thread's column
+  // surface factor i of this cell, or the context constant `k` when the kernel runs without per-cell parameters
+  __device__ __forceinline__ raw par(int i, raw k) const {
+    if constexpr (PAR) return get(kSCount + i); else return k;
+  }
   __device__ __forceinline__ raw get(int i) const {
     raw x;
     if constexpr (sizeof(raw) == 8) asm volatile("ld.volatile.shared.f64 %0, [%1];" : "=d"(x) : "r"(base + i * BLOCK * 8));
@@ -250,8 +262,8 @@ __device__ __forceinline__ Num<P> clear_sky(const Consts<typename P::raw>& k, co
   } else {
     e_tau = nexp(fmadd(b_sa, M_opt, a_sa)); e_gam = nexp(fmadd(b_s, M_opt, a_s));
   }
-  const R tau = nmin(relu(e_tau - R(k.dust)), R(1.0));
-  const R gam_s = (R(1.0) - e_gam) + R(k.dust);
+  const R tau = nmin(relu(e_tau - R(s.par(kPDust, k.dust))), R(1.0));
+  const R gam_s = (R(1.0) - e_gam) + R(s.par(kPDust, k.dust));
   // ET_Radiation_Flux solar_funcs.py:391-412 ; ET_Radiation_Flux_Slope :866-887
   const R isc_e0(tr.isc_e0);
   // (cos_d cos_lat) cos(wt) + sin_d sin_lat is cos Z itself: the products commute exactly, so the lean path reuses it
@@ -340,7 +352,8 @@ __device__ __forceinline__ void lean_forcing(const Consts<double>& k, const Time
   d.v[kD_Xb] = cq * fma(-RH, es_zero, e_air);
   d.v[kD_Tdew] = T_dew; d.v[kD_RH] = RH;
   // -- update_em_air :1167-1180 (Brutsaert), incoming longwave :1234
-  const double em_air = fma(k.emis_a * fm::root7((e_air * kLit.c01) * rTK), k.emis_b, k.canopy);
+  const double em_air = fma(s.par(kPEmisA, k.emis_a) * fm::root7((e_air * kLit.c01) * rTK), s.par(kPEmisB, k.emis_b),
+                            s.par(kPCanopy, k.canopy));
   const double tk2 = T_K * T_K;
   d.v[kD_LWin] = (em_air * k.sigma) * (tk2 * tk2);
   // -- update_julian_day :990-1004 ; True_Solar_Noon solar_funcs.py:1471 ; Clear_Sky_Radiation solar_funcs.py:894-953
@@ -361,8 +374,8 @@ __device__ __forceinline__ void lean_forcing(const Consts<double>& k, const Time
                           fma(fma(-kLit.s_b1, W_p, kLit.s_b0), M_opt, fma(-kLit.s_a1, W_p, kLit.s_a0))};      // :649-653
     double ey[2];
     fm::exp_tab_n<2>(ex, ey);
-    const double tau = nmin(relu(Num<FastF64>(ey[0] - k.dust)), Num<FastF64>(1.0)).v;
-    const double half_gam = 0.5 * ((1.0 - ey[1]) + k.dust);
+    const double tau = nmin(relu(Num<FastF64>(ey[0] - s.par(kPDust, k.dust))), Num<FastF64>(1.0)).v;
+    const double half_gam = 0.5 * ((1.0 - ey[1]) + s.par(kPDust, k.dust));
     const double K_h = relu(Num<FastF64>(tr.isc_e0 * fma(tr.cos_decl * cos_lat, c_wt, tr.sin_decl * sin_lat))).v;      // :391-412
     const double K_s = relu(Num<FastF64>(tr.isc_e0 * fma(tr.cos_decl * s.get(kSCosEq), c_u, s.get(kSSinEq) * tr.sin_decl))).v;  // :866-887
     const double K_dif = half_gam * K_h;                                                 // :667
@@ -418,7 +431,7 @@ __device__ __forceinline__ void lean_state(const Consts<double>& k, Cell& s, Cel
   const bool stable = top > 0.0;
   const double num = stable ? bot : fma(-10.0, top, bot);
   const double den = stable ? fma(10.0, top, bot) : bot;
-  const double L = fm::log_tab(nmax(R((k.z - h_snow) * k.inv_z0), R(kLit.c001)).v);
+  const double L = fm::log_tab(nmax(R((k.z - h_snow) * s.par(kPInvZ0, k.inv_z0)), R(kLit.c001)).v);
   const double uk2 = uz * k.kappa2, LL = L * L;
   const double Dh = (uk2 * num) * fm::rcp3(LL * den);
   const double Qh = (k.rho_cp_air * Dh) * dT;                                   // :744-745
@@ -437,7 +450,7 @@ __device__ __forceinline__ void lean_state(const Consts<double>& k, Cell& s, Cel
   const double Qn_SW = fma(albedo, d.get(kD_B), d.get(kD_A)) * (1.0 - albedo);
   const double T_surf_K = T_surf + kLit.kelvin, ts2 = T_surf_K * T_surf_K;
   const double LW_in = d.get(kD_LWin);
-  const double LW_out = fma(k.one_m_es, LW_in, k.es_sigma * (ts2 * ts2));
+  const double LW_out = fma(s.par(kPOneMEs, k.one_m_es), LW_in, s.par(kPEsSigma, k.es_sigma) * (ts2 * ts2));
   const double Qn_LW = LW_in - LW_out;
   const double Q_sum = ((Qn_SW + Qn_LW) + Qh) + Qe;
   // -- snow: update_snow_meltrate :1364-1368, enforce_max_snow_meltrate :1465
@@ -502,7 +515,9 @@ struct ColumnTerms {
 
 // the forcing-only terms of one column and timestep; `sane` as in the melt kernel's fast-path test (otherwise the
 // kernel takes the strict step from the raw forcings and none of the terms is read)
-template <class P>
+// PAR (per-cell parameters bound): the emissivity and longwave slots carry the parameter-free factors x**(1/7) and
+// T_K**4 instead, from which the melt kernel forms em_air and LW_in with the cell's parameters (same operations)
+template <class P, bool PAR = false>
 __device__ __forceinline__ void column_terms_eval(const Consts<double>& k, double Pp, double T_air_, double P_air_, double q_,
                                                   double uz, bool sane, double* out) {
   using R = Num<P>;
@@ -537,8 +552,14 @@ __device__ __forceinline__ void column_terms_eval(const Consts<double>& k, doubl
     const R W_p = LIT(wp_a, 1.12) * R(ey2[0]);
     const R es_dew = LIT(esat10, 6.11) * R(ey2[1]);
     const R x = (e_air * LIT(c01, 0.1)) * rTK;
-    const R em_air = fmadd(R(k.emis_a) * R(fm::root7(x.v)), R(k.emis_b), R(k.canopy));
-    const R LW_in = (em_air * R(k.sigma)) * npow4(T_K);
+    R em_air, LW_in;
+    if constexpr (PAR) {
+      em_air = R(fm::root7(x.v));
+      LW_in = npow4(T_K);
+    } else {
+      em_air = fmadd(R(k.emis_a) * R(fm::root7(x.v)), R(k.emis_b), R(k.canopy));
+      LW_in = (em_air * R(k.sigma)) * npow4(T_K);
+    }
     R T_wb;
     bool stull_fast;
     if constexpr (TFG_WETBULB_TABLE) stull_fast = (RH >= 0.046875) && (RH <= 2.0);
@@ -564,7 +585,7 @@ __device__ __forceinline__ void column_terms_eval(const Consts<double>& k, doubl
 // strict per-cell step, operation for operation), SATTERLUND configurations included.  There is no "sane" test in this
 // mode -- a missing value poisons the column's terms exactly as it poisons every cell of the column in the per-cell
 // step.  Slot kCtRTK carries e_sat(0 degC) here (the strict step has no use for 1/T_K).
-template <class P>
+template <class P, bool PAR = false>
 __device__ __forceinline__ void column_terms_eval_strict(const Consts<double>& k, double Pp, double T_air_, double P_air_,
                                                          double q_, double uz, double* out) {
   using R = Num<P>;
@@ -581,15 +602,20 @@ __device__ __forceinline__ void column_terms_eval_strict(const Consts<double>& k
   double zero = 0.0;
   asm volatile("" : "+d"(zero));   // opaque: e_sat(0) goes through the device functions like the per-cell step's, not the compiler's folding
   const R es_dew = e_sat_mbar<P>(k, T_dew), es_zero = e_sat_mbar<P>(k, R(zero));
-  R em_air;                                                        // :1167-1192
+  R em_air, LW_in;                                                 // :1167-1192
   if (!k.satterlund) {
     const R x = divk(e_air, 10.0) / T_K;
-    const R term1 = R(k.emis_a) * npow(x, R(k.one_seventh));
-    em_air = fmadd(term1, R(k.emis_b), R(k.canopy));
+    if constexpr (PAR) {   // the parameter-free factors, as in column_terms_eval
+      em_air = npow(x, R(k.one_seventh));
+    } else {
+      const R term1 = R(k.emis_a) * npow(x, R(k.one_seventh));
+      em_air = fmadd(term1, R(k.emis_b), R(k.canopy));
+    }
   } else {
     em_air = R(1.08) * (R(1.0) - nexp(R(-1.0) * npow(e_air, divk(T_K, 2016.0))));
   }
-  const R LW_in = (em_air * R(k.sigma)) * npow4(T_K);              // :1234
+  if (PAR && !k.satterlund) LW_in = npow4(T_K);
+  else LW_in = (em_air * R(k.sigma)) * npow4(T_K);                 // :1234
   const R T_wb = ((((T_air * natan(LIT(st_a, 0.151977) * nsqrt(RH + LIT(st_b, 8.313659)))) + natan(T_air + RH)) -
                    natan(RH - LIT(st_c, 1.676331))) +
                   ((LIT(st_d, 0.00391838) * npow15(RH)) * natan(LIT(st_e, 0.023101) * RH))) -
@@ -654,7 +680,7 @@ __device__ __forceinline__ void cell_step(const Consts<typename P::raw>& k, cons
     rTK = R(pre.rTK); e_air = R(pre.e_air); RH = R(pre.RH); T_dew = R(pre.T_dew);
     double2 late0 = make_double2(0.0, 0.0);   // W_p, e_sat(T_dew): consumed at the end of this block
     if constexpr (TFG_CT_HOIST) late0 = __ldg(reinterpret_cast<const double2*>(pre.line + kCtWp));
-    const double lx1[1] = {nmax((R(k.z) - h_snow) * R(k.inv_z0), LIT(c001, 0.01)).v};
+    const double lx1[1] = {nmax((R(k.z) - h_snow) * R(s.par(kPInvZ0, k.inv_z0)), LIT(c001, 0.01)).v};
     double ly1[1];
     fm::log_tab_n<1>(lx1, ly1);
     const R L(ly1[0]);
@@ -713,7 +739,7 @@ __device__ __forceinline__ void cell_step(const Consts<typename P::raw>& k, cons
     else ex_p0 = -((R(s.get(kSaElev)) * R(k.inv_rstar)) * rTK);
     const double ex2[2] = {ex_p0.v, (-((LIT(mag_a, 17.3) * T_air) * R(rc3[2]))).v};
     const double lx2[2] = {(e_air * LIT(inv_dew_a, 0.1636098885816659)).v,
-                           nmax((R(k.z) - h_snow) * R(k.inv_z0), LIT(c001, 0.01)).v};
+                           nmax((R(k.z) - h_snow) * R(s.par(kPInvZ0, k.inv_z0)), LIT(c001, 0.01)).v};
     double ey2[2], ly2[2];
     if constexpr (!(TFG_EXP5 && TFG_ALBEDO_EARLY)) fm::exp_tab_n<2>(ex2, ey2);
     fm::log_tab_n<2>(lx2, ly2);
@@ -786,7 +812,7 @@ __device__ __forceinline__ void cell_step(const Consts<typename P::raw>& k, cons
     R bot = (uz * uz) * T_K;
     bot = sel(bot == 0.0, R(0.01), bot);
     Ri = top / bot;
-    const R zr = (R(k.z) - h_snow) / R(k.z0_air);                                            // :670-733
+    const R zr = (R(k.z) - h_snow) / R(s.par(kPZ0, k.z0_air));                               // :670-733
     const R arg = R(k.kappa) / nlog(nmax(zr, R(0.01)));
     Dn = uz * (arg * arg);
     if (T_air == T_surf) Dh = Dn;
@@ -820,7 +846,8 @@ __device__ __forceinline__ void cell_step(const Consts<typename P::raw>& k, cons
     Ri = top / bot;
     // ---- update_bulk_aero_conductance :670-733
     R zr;
-    if constexpr (P::strict) zr = (R(k.z) - h_snow) / R(k.z0_air); else zr = (R(k.z) - h_snow) * R(k.inv_z0);
+    if constexpr (P::strict) zr = (R(k.z) - h_snow) / R(s.par(kPZ0, k.z0_air));
+    else zr = (R(k.z) - h_snow) * R(s.par(kPInvZ0, k.inv_z0));
     const R arg = R(k.kappa) / nlog(nmax(zr, R(0.01)));
     Dn = uz * (arg * arg);
     if (T_air == T_surf) Dh = Dn;
@@ -866,27 +893,38 @@ __device__ __forceinline__ void cell_step(const Consts<typename P::raw>& k, cons
   const R Qn_SW = K_cs * (R(1.0) - albedo);
   // ---- update_em_air :1167-1192
   R em_air;
-  if constexpr (Pre::on) {
+  if constexpr (Pre::on && Cell::kPar) {
+    // per-cell parameters: the line holds the parameter-free factor (x**(1/7)) unless SATTERLUND, which takes none
+    if (P::lean || !k.satterlund)
+      em_air = fmadd(R(s.par(kPEmisA, k.emis_a)) * R(pre.get(kCtEmAir)), R(s.par(kPEmisB, k.emis_b)), R(s.par(kPCanopy, k.canopy)));
+    else
+      em_air = R(pre.get(kCtEmAir));
+  } else if constexpr (Pre::on) {
     em_air = R(pre.get(kCtEmAir));   // recording only
   } else if (P::lean || !k.satterlund) {
     R x;
     if constexpr (P::lean) x = (e_air * LIT(c01, 0.1)) * rTK; else x = divk(e_air, 10.0) / T_K;
     R term1;
-    if constexpr (P::lean && TFG_FUSE_ROOT7) term1 = R(k.emis_a) * R(root7_pre);
-    else if constexpr (P::lean) term1 = R(k.emis_a) * R(fm::root7(x.v));   // x > 0 on the sane path
-    else term1 = R(k.emis_a) * npow(x, R(k.one_seventh));
-    em_air = fmadd(term1, R(k.emis_b), R(k.canopy));
+    if constexpr (P::lean && TFG_FUSE_ROOT7) term1 = R(s.par(kPEmisA, k.emis_a)) * R(root7_pre);
+    else if constexpr (P::lean) term1 = R(s.par(kPEmisA, k.emis_a)) * R(fm::root7(x.v));   // x > 0 on the sane path
+    else term1 = R(s.par(kPEmisA, k.emis_a)) * npow(x, R(k.one_seventh));
+    em_air = fmadd(term1, R(s.par(kPEmisB, k.emis_b)), R(s.par(kPCanopy, k.canopy)));
   } else {
     em_air = R(1.08) * (R(1.0) - nexp(R(-1.0) * npow(e_air, divk(T_K, 2016.0))));
   }
   // ---- update_net_longwave_radiation :1231-1248
   const R T_surf_K = T_surf + LIT(kelvin, 273.15);
   R LW_in;
-  if constexpr (Pre::on && TFG_CT_HOIST) LW_in = R(late1.x);
+  if constexpr (Pre::on && Cell::kPar) {   // the line holds T_K**4 unless SATTERLUND (then LW_in itself)
+    const R line = TFG_CT_HOIST ? R(late1.x) : R(pre.get(kCtLWin));
+    if (P::lean || !k.satterlund) LW_in = (em_air * R(k.sigma)) * line;
+    else LW_in = line;
+  }
+  else if constexpr (Pre::on && TFG_CT_HOIST) LW_in = R(late1.x);
   else if constexpr (Pre::on) LW_in = R(pre.get(kCtLWin));
   else LW_in = (em_air * R(k.sigma)) * npow4(T_K);
-  R LW_out = R(k.es_sigma) * npow4(T_surf_K);
-  LW_out = fmadd(R(k.one_m_es), LW_in, LW_out);
+  R LW_out = R(s.par(kPEsSigma, k.es_sigma)) * npow4(T_surf_K);
+  LW_out = fmadd(R(s.par(kPOneMEs, k.one_m_es)), LW_in, LW_out);
   const R Qn_LW = LW_in - LW_out;
   // ---- update_net_energy_flux :1314  (Qa = Qc = 0, :312-313)
   R Q_sum = ((Qn_SW + Qn_LW) + Qh) + Qe;

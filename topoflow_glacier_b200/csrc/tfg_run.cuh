@@ -79,6 +79,7 @@ struct RunParams {
   alignas(16) Consts<raw> k;
   const raw* col_terms;        // optional [n_steps][n_cols][kCtCount] (fast float64 mode, forcing map bound): the column
                                // terms of this launch (column_terms_kernel); the kernel then does not read `forcing`
+  const raw* cell_par;         // optional [kPCount][n_cells] per-cell surface factors (tfg_bind_cell_params)
 };
 
 template <class raw> __device__ __forceinline__ raw ld_stream(const raw* p) { return __ldcs(p); }
@@ -181,7 +182,7 @@ __device__ __forceinline__ void agg_add_exact(long long* acc, double v, double u
   if (b) atomicAdd(reinterpret_cast<unsigned long long*>(acc) + 1, (unsigned long long)b);
 }
 
-template <class P, bool REC, bool AGG, bool VOL, bool TMA = false, bool PRE = false>
+template <class P, bool REC, bool AGG, bool VOL, bool TMA = false, bool PRE = false, bool PAR = false>
 __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f32 ? TFG_MIN_BLOCKS_F32 : TFG_MIN_BLOCKS)) run_kernel(const __grid_constant__ RunParams<typename P::raw> p) {
   using raw = typename P::raw;
   using R = Num<P>;
@@ -197,10 +198,17 @@ __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f3
   }
   // per-cell constants + diagnostic integrals live in shared memory (one column per thread)
   constexpr bool kSmem = true;  // RegCell (registers) remains available for experiments
-  __shared__ raw sm_cell[kSmem ? kSCount : 1][kBlock];
-  using Cell = typename std::conditional<kSmem, SmemCell<raw, kBlock>, RegCell<raw>>::type;
+  static_assert(kSmem || !PAR, "per-cell parameters live in shared memory");
+  static_assert(!(PAR && TMA), "per-cell parameters run the register-prefetch kernel");
+  // PAR: the per-cell surface factors in kPCount more columns (only in these instantiations: the others keep their footprint)
+  __shared__ raw sm_cell[kSmem ? kSCount + (PAR ? kPCount : 0) : 1][kBlock];
+  using Cell = typename std::conditional<kSmem, SmemCell<raw, kBlock, PAR>, RegCell<raw>>::type;
   Cell s;
   if constexpr (kSmem) s.base = (unsigned)__cvta_generic_to_shared(&sm_cell[0][threadIdx.x]);
+  if constexpr (PAR) {
+#pragma unroll
+    for (int i = 0; i < kPCount; ++i) s.set(kSCount + i, __ldg(p.cell_par + (int64_t)i * p.n_cells + c));
+  }
   s.set(kSaElev, __ldg(p.a_elev + c)); s.set(kSSinLat, __ldg(p.sin_lat + c)); s.set(kSCosLat, __ldg(p.cos_lat + c));
   s.set(kSNegTanLat, __ldg(p.neg_tan_lat + c)); s.set(kSSinEq, __ldg(p.sin_eq + c)); s.set(kSCosEq, __ldg(p.cos_eq + c));
   s.set(kSNegTanEq, __ldg(p.neg_tan_eq + c)); s.set(kSDlon, __ldg(p.dlon + c)); s.set(kSTNoon, __ldg(p.t_noon + c));
@@ -567,7 +575,7 @@ __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f3
 // Column terms of one launch: thread = (timestep, column) of the forcing block [n_steps][5][n_cols]; writes one line of
 // kCtCount doubles (see tfg_physics.cuh).  Compiled in the fast translation unit, with the melt kernel's own device
 // functions, so the values equal what the per-cell step computes (tests: mapped forcing == replicated forcing, bit for bit).
-template <class P>
+template <class P, bool PAR = false>
 __global__ void __launch_bounds__(256) column_terms_kernel(const double* __restrict__ forcing, double* __restrict__ out,
                                                            int32_t n_steps, int64_t n_cols, const Consts<double> k) {
   if constexpr (P::lean) {
@@ -580,57 +588,69 @@ __global__ void __launch_bounds__(256) column_terms_kernel(const double* __restr
   const int64_t t = idx / n_cols, col = idx - t * n_cols;
   const double* f = forcing + t * (TFG_N_FORCING * n_cols) + col;
   const double f0 = f[0], f1 = f[n_cols], f2 = f[2 * n_cols], f3 = f[3 * n_cols], f4 = f[4 * n_cols];
-  if constexpr (P::lean) column_terms_eval<P>(k, f0, f1, f2, f3, f4, forcings_sane(f0, f1, f2, f3, f4), out + idx * kCtCount);
-  else column_terms_eval_strict<P>(k, f0, f1, f2, f3, f4, out + idx * kCtCount);
+  if constexpr (P::lean) column_terms_eval<P, PAR>(k, f0, f1, f2, f3, f4, forcings_sane(f0, f1, f2, f3, f4), out + idx * kCtCount);
+  else column_terms_eval_strict<P, PAR>(k, f0, f1, f2, f3, f4, out + idx * kCtCount);
 }
 
+// par: the melt kernel runs with per-cell parameters, so the line carries their parameter-free factors (column_terms_eval)
 template <class P>
 cudaError_t launch_column_terms(const double* forcing, double* out, int32_t n_steps, int64_t n_cols, const Consts<double>& k,
-                                cudaStream_t stream) {
+                                bool par, cudaStream_t stream) {
   const int64_t total = (int64_t)n_steps * n_cols;
-  column_terms_kernel<P><<<(unsigned)((total + 255) / 256), 256, P::lean ? fm::kTabDoubles * sizeof(double) : 0, stream>>>(forcing, out, n_steps,
-                                                                                                           n_cols, k);
+  const unsigned grid = (unsigned)((total + 255) / 256);
+  const size_t dyn = P::lean ? fm::kTabDoubles * sizeof(double) : 0;
+  if (par) column_terms_kernel<P, true><<<grid, 256, dyn, stream>>>(forcing, out, n_steps, n_cols, k);
+  else column_terms_kernel<P><<<grid, 256, dyn, stream>>>(forcing, out, n_steps, n_cols, k);
   return cudaGetLastError();
 }
 
-template <class P>
-cudaError_t launch_run(const RunParams<typename P::raw>& p, bool rec, bool agg, bool vol, cudaStream_t stream) {
+template <class P, bool PAR>
+cudaError_t launch_run_as(const RunParams<typename P::raw>& p, bool rec, bool agg, bool vol, cudaStream_t stream) {
   const unsigned grid = (unsigned)((p.n_cells + kBlock - 1) / kBlock);
-  // TMA staging needs whole blocks and 16-byte aligned rows; otherwise the register-prefetch kernel runs
-  const bool tma = p.use_tma && !rec && !p.forcing_col && (p.n_cells % kBlock == 0) && p.n_steps >= 2 &&
+  // TMA staging needs whole blocks and 16-byte aligned rows; otherwise the register-prefetch kernel runs (always with
+  // per-cell parameters, as with a forcing map)
+  const bool tma = !PAR && p.use_tma && !rec && !p.forcing_col && (p.n_cells % kBlock == 0) && p.n_steps >= 2 &&
                    ((reinterpret_cast<uintptr_t>(p.forcing) & 15) == 0) &&
                    ((p.n_cells * sizeof(typename P::raw)) % 16 == 0);
   const size_t dyn = P::lean ? fm::kTabDoubles * sizeof(double) : 0;
   if constexpr (!P::f32) {
     if (p.col_terms != nullptr) {  // column terms bound (forcing map): the kernel reads them instead of the forcing block
-      if (rec) run_kernel<P, true, true, true, false, true><<<grid, kBlock, dyn, stream>>>(p);
-      else if (agg && vol) run_kernel<P, false, true, true, false, true><<<grid, kBlock, dyn, stream>>>(p);
-      else if (agg) run_kernel<P, false, true, false, false, true><<<grid, kBlock, dyn, stream>>>(p);
-      else if (vol) run_kernel<P, false, false, true, false, true><<<grid, kBlock, dyn, stream>>>(p);
-      else run_kernel<P, false, false, false, false, true><<<grid, kBlock, dyn, stream>>>(p);
+      if (rec) run_kernel<P, true, true, true, false, true, PAR><<<grid, kBlock, dyn, stream>>>(p);
+      else if (agg && vol) run_kernel<P, false, true, true, false, true, PAR><<<grid, kBlock, dyn, stream>>>(p);
+      else if (agg) run_kernel<P, false, true, false, false, true, PAR><<<grid, kBlock, dyn, stream>>>(p);
+      else if (vol) run_kernel<P, false, false, true, false, true, PAR><<<grid, kBlock, dyn, stream>>>(p);
+      else run_kernel<P, false, false, false, false, true, PAR><<<grid, kBlock, dyn, stream>>>(p);
       return cudaGetLastError();
     }
   }
-  if (rec) run_kernel<P, true, true, true><<<grid, kBlock, dyn, stream>>>(p);
+  if (rec) run_kernel<P, true, true, true, false, false, PAR><<<grid, kBlock, dyn, stream>>>(p);
   else if (tma) {
-    if (agg && vol) run_kernel<P, false, true, true, true><<<grid, kBlock, dyn, stream>>>(p);
-    else if (agg) run_kernel<P, false, true, false, true><<<grid, kBlock, dyn, stream>>>(p);
-    else if (vol) run_kernel<P, false, false, true, true><<<grid, kBlock, dyn, stream>>>(p);
-    else run_kernel<P, false, false, false, true><<<grid, kBlock, dyn, stream>>>(p);
+    if constexpr (!PAR) {
+      if (agg && vol) run_kernel<P, false, true, true, true><<<grid, kBlock, dyn, stream>>>(p);
+      else if (agg) run_kernel<P, false, true, false, true><<<grid, kBlock, dyn, stream>>>(p);
+      else if (vol) run_kernel<P, false, false, true, true><<<grid, kBlock, dyn, stream>>>(p);
+      else run_kernel<P, false, false, false, true><<<grid, kBlock, dyn, stream>>>(p);
+    }
   }
-  else if (agg && vol) run_kernel<P, false, true, true><<<grid, kBlock, dyn, stream>>>(p);
-  else if (agg) run_kernel<P, false, true, false><<<grid, kBlock, dyn, stream>>>(p);
-  else if (vol) run_kernel<P, false, false, true><<<grid, kBlock, dyn, stream>>>(p);
-  else run_kernel<P, false, false, false><<<grid, kBlock, dyn, stream>>>(p);
+  else if (agg && vol) run_kernel<P, false, true, true, false, false, PAR><<<grid, kBlock, dyn, stream>>>(p);
+  else if (agg) run_kernel<P, false, true, false, false, false, PAR><<<grid, kBlock, dyn, stream>>>(p);
+  else if (vol) run_kernel<P, false, false, true, false, false, PAR><<<grid, kBlock, dyn, stream>>>(p);
+  else run_kernel<P, false, false, false, false, false, PAR><<<grid, kBlock, dyn, stream>>>(p);
   return cudaGetLastError();
+}
+
+// per-cell surface parameters bound (tfg_bind_cell_params): the PAR instantiations, chosen from the input
+template <class P>
+cudaError_t launch_run(const RunParams<typename P::raw>& p, bool rec, bool agg, bool vol, cudaStream_t stream) {
+  return p.cell_par != nullptr ? launch_run_as<P, true>(p, rec, agg, vol, stream) : launch_run_as<P, false>(p, rec, agg, vol, stream);
 }
 
 cudaError_t launch_run_strict(const RunParams<double>& p, bool rec, bool agg, bool vol, cudaStream_t stream);
 cudaError_t launch_run_fast(const RunParams<double>& p, bool rec, bool agg, bool vol, cudaStream_t stream);
 cudaError_t launch_run_f32(const RunParams<float>& p, bool rec, bool agg, bool vol, cudaStream_t stream);
 cudaError_t launch_column_terms_fast(const double* forcing, double* out, int32_t n_steps, int64_t n_cols, const Consts<double>& k,
-                                     cudaStream_t stream);
+                                     bool par, cudaStream_t stream);
 cudaError_t launch_column_terms_strict(const double* forcing, double* out, int32_t n_steps, int64_t n_cols, const Consts<double>& k,
-                                       cudaStream_t stream);
+                                       bool par, cudaStream_t stream);
 
 }  // namespace tfg

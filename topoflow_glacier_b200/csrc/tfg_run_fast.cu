@@ -31,7 +31,7 @@ cudaError_t launch_run_fast(const RunParams<double>& p, bool rec, bool agg, bool
 #endif
 }
 cudaError_t launch_column_terms_fast(const double* forcing, double* out, int32_t n_steps, int64_t n_cols, const Consts<double>& k,
-                                     cudaStream_t stream) {
-  return launch_column_terms<FastF64>(forcing, out, n_steps, n_cols, k, stream);
+                                     bool par, cudaStream_t stream) {
+  return launch_column_terms<FastF64>(forcing, out, n_steps, n_cols, k, par, stream);
 }
 }  // namespace tfg

@@ -18,7 +18,7 @@ import pandas as pd
 import torch
 
 from . import _lib
-from .config import KERNEL_CONSTANTS
+from .config import CELL_PARAM_KEYS, KERNEL_CONSTANTS, check_cell_params
 from .statics import cell_tables
 from .timebase import parse_start, time_tables, utc_offsets
 
@@ -52,6 +52,10 @@ class MeltEngine:
         one catchment share the catchment's forcing series, so forcing is ``[T, 5, n_forcing_cols]`` instead of
         ``[T, 5, N]`` -- nothing is replicated per cell on the host or over PCIe (``tfg_bind_forcing_map``)
     basin_id : per-cell int32 basin index in ``[0, n_basin)`` or None
+    cell_params : optional mapping of any of ``config.CELL_PARAM_KEYS`` (``dust_atten, canopy_factor, cloud_factor,
+        z0_air, em_surf``) to per-cell ``[N]`` arrays or device tensors: every cell runs with its own values (a
+        parameter ensemble, e.g. one calibration candidate per cell); keys it does not name take the value of
+        ``consts``.  See ``set_cell_params``.
     mode : ``"f64"`` (strict), ``"f64_fast"`` or ``"f32"``
     horizon_steps : number of steps the host time tables are prepared for (extended on demand)
     """
@@ -61,7 +65,7 @@ class MeltEngine:
                  basin_id: Optional[np.ndarray] = None, n_basin: int = 0, mode: str = "f64", device: int = 0,
                  horizon_steps: int = 24 * 366, diag_integrals: bool = True, device_statics: Optional[dict] = None,
                  tma_staging: Optional[bool] = None, forcing_index=None, n_forcing_cols: Optional[int] = None,
-                 column_terms: Optional[bool] = None):
+                 column_terms: Optional[bool] = None, cell_params: Optional[Mapping] = None):
         self.lib = _lib.load()
         self.device = _require_cuda(device)
         self.mode = _lib.MODE_NAMES[mode] if isinstance(mode, str) else int(mode)
@@ -116,6 +120,9 @@ class MeltEngine:
             self.tz_idx = None if tz_idx is None else torch.as_tensor(
                 np.ascontiguousarray(tz_idx, dtype=np.uint8)).to(self.device)
             self._bind_static()
+            self.cell_params = None
+            if cell_params is not None:
+                self.set_cell_params(cell_params)
             self.n_cols, self.forcing_index = N, None
             if forcing_index is not None:
                 self.set_forcing_map(forcing_index, n_forcing_cols, _alloc_inputs=False)
@@ -147,6 +154,33 @@ class MeltEngine:
         s.basin_id = self.basin_id.data_ptr() if self.basin_id is not None else None
         s.tz_idx = self.tz_idx.data_ptr() if self.tz_idx is not None else None
         _lib.check(self.lib.tfg_bind_static(self.ctx, self.N, C.byref(s)), "tfg_bind_static")
+
+    def set_cell_params(self, params: Optional[Mapping]) -> None:
+        """Bind per-cell surface parameters (``None`` unbinds them); may be called between launches.
+
+        ``params`` maps any of ``config.CELL_PARAM_KEYS`` to ``[N]`` arrays or tensors; unnamed keys take the engine's
+        constants.  Values are range-checked with the schema's bounds (``ValueError``).  A key whose values all equal
+        the constant is not bound, and with no key left the engine runs exactly as without parameters.  A calibration
+        loop: ``run``, score, ``set_cell_params(next_candidates)``, ``load_state_dict(initial)``, ``run`` again."""
+        tensors = {k: (v if torch.is_tensor(v) else torch.as_tensor(np.asarray(v, dtype=np.float64)))
+                   .to(self.device, torch.float64).contiguous().reshape(-1) for k, v in (params or {}).items()}
+        bound = {}
+        for k, t in check_cell_params(tensors).items():
+            if t.numel() != self.N:
+                raise ValueError(f"{k}: one value per cell ({self.N}) expected, got {t.numel()}")
+            if not bool((t == self.consts[k]).all()):
+                bound[k] = t
+        with torch.cuda.device(self.device):
+            if not bound:
+                _lib.check(self.lib.tfg_bind_cell_params(self.ctx, None, self.stream_ptr), "tfg_bind_cell_params")
+                self.cell_params = None
+                return
+            p = _lib.CellParams()
+            for k in CELL_PARAM_KEYS:
+                setattr(p, k, bound[k].data_ptr() if k in bound else None)
+            # the library derives its own copy on the current stream and waits for its range check
+            _lib.check(self.lib.tfg_bind_cell_params(self.ctx, C.byref(p), self.stream_ptr), "tfg_bind_cell_params")
+        self.cell_params = bound
 
     def _init_state(self, init):
         """Initial state of reference ``initialize()`` (``:350-395``): depths from the config, albedo 0.3,

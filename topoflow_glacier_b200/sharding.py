@@ -160,12 +160,15 @@ class ShardedMeltEngine:
     ``cells`` is either the mapping of GLOBAL float64 ``[n_total]`` arrays ``MeltEngine`` takes (sliced here), or a
     callable ``(lo, hi) -> mapping`` that produces the shard's arrays (host arrays keyed like ``cells``, or device
     tables keyed like ``tfg_statics`` + ``h0_*``) for grids too large to materialise on every rank; then pass
-    ``n_total``.  ``basin_id`` / ``tz_idx`` / ``forcing_index`` are global arrays (or callables ``(lo, hi)``).
+    ``n_total``.  ``basin_id`` / ``tz_idx`` / ``forcing_index`` are global arrays (or callables ``(lo, hi)``); so is
+    ``cell_params``: a mapping of global per-cell parameter arrays (``MeltEngine(cell_params=...)``), sliced here, or a
+    callable ``(lo, hi) -> mapping`` of the shard's arrays.
     Attribute access falls through to the local ``MeltEngine`` (``state``, ``row``, ``step_index`` ...).
     """
 
     def __init__(self, cells, consts, start_time, *, n_total: Optional[int] = None, basin_id=None, n_basin: int = 0,
-                 tz_idx=None, forcing_index=None, group=None, exact: bool = True, device: Optional[int] = None, **kw):
+                 tz_idx=None, forcing_index=None, cell_params=None, group=None, exact: bool = True,
+                 device: Optional[int] = None, **kw):
         import os
 
         import torch
@@ -192,11 +195,13 @@ class ShardedMeltEngine:
         local = cells(lo, hi) if callable(cells) else {k: np.asarray(v)[lo:hi] for k, v in cells.items()}
         if device is None:
             device = int(os.environ.get("LOCAL_RANK", self.rank)) % max(torch.cuda.device_count(), 1)
+        if cell_params is not None:
+            cell_params = cell_params(lo, hi) if callable(cell_params) else {k: v[lo:hi] for k, v in cell_params.items()}
         dev_tables = "a_elev" in local
         self.exact = bool(exact)
         self.engine = MeltEngine(None if dev_tables else local, consts, start_time, basin_id=part(basin_id),
                                  n_basin=n_basin, tz_idx=part(tz_idx), forcing_index=part(forcing_index), device=device,
-                                 device_statics=local if dev_tables else None, **kw)
+                                 device_statics=local if dev_tables else None, cell_params=cell_params, **kw)
         self._aggs: dict = {}
 
     def __getattr__(self, name):
