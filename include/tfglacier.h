@@ -193,6 +193,37 @@ typedef struct tfg_cell_params {
  * read again afterwards.  A cell whose parameters equal the constants gives the bits of an unbound run.          */
 TFG_API int tfg_bind_cell_params(tfg_ctx* ctx, const tfg_cell_params* p, void* stream);
 
+/* Optional objective: while one is bound, every tfg_run launch compares one BMI output of every cell with an observed
+ * series and adds four float64 sums per cell into `acc`, so that a calibration or sensitivity run scores each
+ * candidate (cell) on the device instead of recording a series per cell-step.
+ *   quantity  TFG_REC_H_SNOW .. TFG_REC_RH (the eight BMI outputs); the value compared for absolute step k is the one
+ *             the record buffer holds for step k (what get_value returns after that update())
+ *   obs       dev float64 [n_obs_steps][n_obs_cols] in every mode; row j belongs to absolute step obs_step0 + j.  A
+ *             non-finite value means "not observed": that step is not scored for the cells reading that column
+ *             (daily observations of an hourly model, a spin-up period).  Steps outside the window are not scored.
+ *   obs_col   dev int32 [n_cells] in [0, n_obs_cols): cell i reads column obs_col[i]; NULL = column i (n_obs_cols
+ *             must then equal n_cells)
+ *   acc       dev float64 [TFG_N_OBJ][n_cells], ACCUMULATED INTO (zero it to start); owned by the caller.  Rows:
+ *             S_s = sum s, S_ss = sum s*s, S_so = sum s*o, S_ee = sum (s-o)*(s-o).  Each scored step runs exactly
+ *             d = s - o; S_s += s; S_ss += s*s; S_so += s*o; S_ee += d*d in float64 (a float32 s widened exactly), each
+ *             operation rounded once, so the sums depend only on the per-step values and their order: they are the
+ *             same bits for any launch split, for the per-step path and for any sharding, and a host float64 loop over
+ *             a recorded series reproduces them.  A cell whose state is NaN is still scored where its observation is
+ *             finite, so its sums become NaN.
+ * NSE, KGE, RMSE and bias follow from the sums and the observations' own moments (topoflow_glacier_b200/objective.py). */
+#define TFG_N_OBJ 4 /* rows of tfg_objective.acc */
+typedef struct tfg_objective {
+  int32_t quantity;                   /* TFG_REC_H_SNOW .. TFG_REC_RH                                          */
+  const double* obs;                  /* dev [n_obs_steps][n_obs_cols]; non-finite = not observed               */
+  int64_t obs_step0, n_obs_steps, n_obs_cols;
+  const int32_t* obs_col;             /* dev [n_cells] in [0, n_obs_cols), or NULL (column = cell)              */
+  double* acc;                        /* dev [TFG_N_OBJ][n_cells], accumulated into                            */
+} tfg_objective;
+/* Bind (o != NULL) or unbind (o == NULL) an objective; call after tfg_bind_static (binding statics again unbinds it).
+ * The host fields are checked, and obs_col's range on the device, on `stream`; the call waits for that check.  On
+ * error nothing is bound and tfg_last_error() names the field.  The arrays are read by every later tfg_run.        */
+TFG_API int tfg_bind_objective(tfg_ctx* ctx, const tfg_objective* o, void* stream);
+
 /* host tables for steps [0, n_steps): rows[n_steps], gmt_offset_hours[n_steps][n_tz]; copied by the library
  * (each launch carries its <= 128 rows in the kernel parameter block); replaces solar.gmt_offset_hours,
  * solar_funcs.py:1616-1637, evaluated on the host                                                 */
@@ -209,6 +240,7 @@ TFG_API int tfg_bind_time(tfg_ctx* ctx, const tfg_time_row* rows, const double* 
  *   basin_agg    dev [n_steps][n_basin][TFG_N_AGG] float64 or NULL: ACCUMULATED INTO (zero it first);
  *                replaces np.sum(...) at :567-568,:1486-1494 and the driver-side `* da_m2`
  *                (examples/run_topoflow_glacier.py:115); int64 fixed-point accumulators under TFG_OPT_EXACT_AGG
+ * With an objective bound (tfg_bind_objective), the steps of [step0, step0 + n_steps) inside its window are scored.
  * n_steps == 1 re-sums the snowfall window exactly every step (the literal update()).          */
 TFG_API int tfg_run(tfg_ctx* ctx, const void* forcing, int64_t step0, int32_t n_steps, void* record, uint64_t record_mask,
             void* basin_agg, int32_t n_basin, void* stream);

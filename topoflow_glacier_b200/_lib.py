@@ -43,6 +43,14 @@ class CellParams(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in CELL_PARAM_FIELDS]
 
 
+N_OBJ = 4  # rows of Objective.acc: S_s, S_ss, S_so, S_ee
+
+
+class Objective(C.Structure):
+    _fields_ = [("quantity", C.c_int32), ("obs", C.c_void_p), ("obs_step0", C.c_int64), ("n_obs_steps", C.c_int64),
+                ("n_obs_cols", C.c_int64), ("obs_col", C.c_void_p), ("acc", C.c_void_p)]
+
+
 class TimeRow(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("clock_hour", "TE", "sin_decl", "cos_decl", "tan_decl", "isc_e0",
                                               "cos_hour", "sin_hour")]
@@ -82,6 +90,7 @@ PROTOTYPES = {
     "tfg_bind_state": (C.c_int, [C.c_void_p, C.POINTER(State)]),
     "tfg_bind_forcing_map": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64]),
     "tfg_bind_cell_params": (C.c_int, [C.c_void_p, C.POINTER(CellParams), C.c_void_p]),
+    "tfg_bind_objective": (C.c_int, [C.c_void_p, C.POINTER(Objective), C.c_void_p]),
     "tfg_bind_window_carry": (C.c_int, [C.c_void_p, C.c_void_p]),
     "tfg_bind_mass_residual": (C.c_int, [C.c_void_p, C.c_void_p]),
     "tfg_bind_time": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),

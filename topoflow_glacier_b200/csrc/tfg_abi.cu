@@ -58,6 +58,9 @@ struct tfg_ctx {
   size_t cell_par_bytes = 0;
   int* cell_par_bad = nullptr;           // device flags of tfg_bind_cell_params' range check (owned)
   bool have_cell_par = false;            // tfg_bind_cell_params: the scratch holds this context's factors
+  tfg_objective obj{};                   // tfg_bind_objective (caller's arrays)
+  bool have_obj = false;
+  int* obj_bad = nullptr;                // device flag of tfg_bind_objective's range check of obs_col (owned)
 };
 
 namespace {
@@ -204,6 +207,21 @@ tfg::RunParams<raw> make_params(const tfg_ctx* x, const void* forcing, int64_t s
   p.n_basin = n_basin;
   p.k = derive<raw>(x->c);
   p.cell_par = x->have_cell_par ? static_cast<const raw*>(x->cell_par) : nullptr;
+  // objective: the scored part of [step0, step0 + n_steps) is its intersection with the observation window; a launch
+  // outside the window leaves obj_acc NULL and runs the kernels without an objective
+  if (x->have_obj) {
+    const tfg_objective& o = x->obj;
+    const int64_t lo = std::max<int64_t>(step0, o.obs_step0), hi = std::min<int64_t>(step0 + n_steps, o.obs_step0 + o.n_obs_steps);
+    if (lo < hi) {
+      p.obj_acc = o.acc;
+      p.obj_obs = o.obs + (lo - o.obs_step0) * o.n_obs_cols;
+      p.obj_col = o.obs_col;
+      p.obj_ncols = o.n_obs_cols;
+      p.obj_t_lo = (int32_t)(lo - step0);
+      p.obj_t_hi = (int32_t)(hi - step0);
+      p.obj_quantity = o.quantity;
+    }
+  }
   return p;
 }
 
@@ -230,6 +248,12 @@ __global__ void cell_params_kernel(const tfg_cell_params in, const tfg_constants
     if (f32) static_cast<float*>(out)[r * N + i] = (float)f[r];
     else static_cast<double*>(out)[r * N + i] = f[r];
   }
+}
+
+// ---- objective (tfg_bind_objective): *bad = 1 if an observation column index is outside [0, n_cols) -------------
+__global__ void obs_col_check_kernel(const int32_t* col, int64_t N, int64_t n_cols, int* bad) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < N && !(col[i] >= 0 && (int64_t)col[i] < n_cols)) atomicOr(bad, 1);
 }
 
 // ---- K2: raw met columns -> live forcings (examples/run_topoflow_glacier.py:40-73) -------------------
@@ -386,6 +410,7 @@ void tfg_destroy(tfg_ctx* x) {
   if (x->col_terms) cudaFree(x->col_terms);
   if (x->cell_par) cudaFree(x->cell_par);
   if (x->cell_par_bad) cudaFree(x->cell_par_bad);
+  if (x->obj_bad) cudaFree(x->obj_bad);
   delete x;
 }
 
@@ -423,6 +448,7 @@ int tfg_bind_static(tfg_ctx* x, int64_t n_cells, const tfg_statics* s) {
   x->n_cells = n_cells;
   x->have_static = true;
   x->have_cell_par = false;  // sized for the old cell count: bind again
+  x->have_obj = false;       // likewise the objective's per-cell arrays
   return 0;
 }
 
@@ -461,6 +487,39 @@ int tfg_bind_cell_params(tfg_ctx* x, const tfg_cell_params* p, void* stream) {
     return fail(m.c_str());
   }
   x->have_cell_par = true;
+  return 0;
+}
+
+int tfg_bind_objective(tfg_ctx* x, const tfg_objective* o, void* stream) {
+  if (!x) return fail("tfg_bind_objective: NULL context");
+  x->have_obj = false;
+  if (!o) return 0;
+#if defined(TFG_LEAN_W2) || TFG_WS || TFG_PIPELINE || TFG_SPLIT_STEP
+  return fail("tfg_bind_objective: this build runs an experimental kernel variant, which has no objective");
+#endif
+  if (!x->have_static) return fail("tfg_bind_objective: call after tfg_bind_static");
+  if (o->quantity < TFG_REC_H_SNOW || o->quantity > TFG_REC_RH)
+    return fail("tfg_bind_objective: quantity must be one of the eight BMI outputs, TFG_REC_H_SNOW .. TFG_REC_RH (0-7)");
+  if (!o->obs) return fail("tfg_bind_objective: obs is NULL");
+  if (!o->acc) return fail("tfg_bind_objective: acc is NULL");
+  if (o->n_obs_steps <= 0) return fail("tfg_bind_objective: n_obs_steps must be > 0");
+  if (o->n_obs_cols <= 0) return fail("tfg_bind_objective: n_obs_cols must be > 0");
+  if (!o->obs_col && o->n_obs_cols != x->n_cells)
+    return fail("tfg_bind_objective: n_obs_cols must equal n_cells when obs_col is NULL (column = cell)");
+  if (o->obs_col) {
+    TFG_CUDA(cudaSetDevice(x->device));
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (!x->obj_bad) TFG_CUDA(cudaMalloc(&x->obj_bad, sizeof(int)));
+    TFG_CUDA(cudaMemsetAsync(x->obj_bad, 0, sizeof(int), s));
+    obs_col_check_kernel<<<(unsigned)((x->n_cells + 255) / 256), 256, 0, s>>>(o->obs_col, x->n_cells, o->n_obs_cols, x->obj_bad);
+    TFG_CUDA(cudaGetLastError());
+    int bad = 0;
+    TFG_CUDA(cudaMemcpyAsync(&bad, x->obj_bad, sizeof(int), cudaMemcpyDeviceToHost, s));
+    TFG_CUDA(cudaStreamSynchronize(s));
+    if (bad) return fail("tfg_bind_objective: obs_col has entries outside [0, n_obs_cols)");
+  }
+  x->obj = *o;
+  x->have_obj = true;
   return 0;
 }
 

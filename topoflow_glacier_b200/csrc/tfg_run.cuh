@@ -80,6 +80,13 @@ struct RunParams {
   const raw* col_terms;        // optional [n_steps][n_cols][kCtCount] (fast float64 mode, forcing map bound): the column
                                // terms of this launch (column_terms_kernel); the kernel then does not read `forcing`
   const raw* cell_par;         // optional [kPCount][n_cells] per-cell surface factors (tfg_bind_cell_params)
+  // objective (tfg_bind_objective): local steps [obj_t_lo, obj_t_hi) of this launch are scored; obj_obs is the
+  // observation row of local step obj_t_lo.  obj_acc == nullptr: no objective (the OBJ instantiations are not chosen)
+  double* obj_acc;             // [TFG_N_OBJ][n_cells], accumulated into
+  const double* obj_obs;       // [obj_t_hi - obj_t_lo][obj_ncols] (rows of this launch)
+  const int32_t* obj_col;      // [n_cells] or nullptr (column = cell)
+  int64_t obj_ncols;
+  int32_t obj_t_lo, obj_t_hi, obj_quantity;
 };
 
 template <class raw> __device__ __forceinline__ raw ld_stream(const raw* p) { return __ldcs(p); }
@@ -182,7 +189,21 @@ __device__ __forceinline__ void agg_add_exact(long long* acc, double v, double u
   if (b) atomicAdd(reinterpret_cast<unsigned long long*>(acc) + 1, (unsigned long long)b);
 }
 
-template <class P, bool REC, bool AGG, bool VOL, bool TMA = false, bool PRE = false, bool PAR = false>
+// The objective's four float64 sums of this thread's cell, one shared-memory column each for the whole launch (as
+// SmemCell keeps the cell constants): volatile accesses, so that they do not occupy registers across the time loop.
+struct ObjSums {
+  unsigned base;  // shared-window address of this thread's column of row 0
+  __device__ __forceinline__ double get(int i) const {
+    double x;
+    asm volatile("ld.volatile.shared.f64 %0, [%1];" : "=d"(x) : "r"(base + i * kBlock * 8));
+    return x;
+  }
+  __device__ __forceinline__ void set(int i, double x) {
+    asm volatile("st.volatile.shared.f64 [%0], %1;" ::"r"(base + i * kBlock * 8), "d"(x));
+  }
+};
+
+template <class P, bool REC, bool AGG, bool VOL, bool TMA = false, bool PRE = false, bool PAR = false, bool OBJ = false>
 __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f32 ? TFG_MIN_BLOCKS_F32 : TFG_MIN_BLOCKS)) run_kernel(const __grid_constant__ RunParams<typename P::raw> p) {
   using raw = typename P::raw;
   using R = Num<P>;
@@ -215,6 +236,16 @@ __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f3
   s.set(kSDa, (TFG_DA_ZERO && !active) ? raw(0) : __ldg(p.da_m2 + c)); s.set(kSTrs, __ldg(p.t_rs + c));
   s.set(kSCB, 0); s.set(kSSB, 0); s.set(kSCB2, 0); s.set(kSSB2, 0);
   s.set(kSaElevR, (raw)(s.get(kSaElev) * p.k.inv_rstar));
+  // OBJ: the objective's sums, float64 in every mode, carried on from the caller's accumulators (one running sum per
+  // quantity over all launches: the result does not depend on how a run is split into launches)
+  static_assert(!(OBJ && TMA), "an objective runs the register-prefetch kernel");
+  __shared__ double sm_obj[OBJ ? TFG_N_OBJ : 1][OBJ ? kBlock : 1];
+  ObjSums osum;
+  if constexpr (OBJ) {
+    osum.base = (unsigned)__cvta_generic_to_shared(&sm_obj[0][threadIdx.x]);
+#pragma unroll
+    for (int i = 0; i < TFG_N_OBJ; ++i) osum.set(i, p.obj_acc[(int64_t)i * p.n_cells + c]);
+  }
   const R lon(__ldg(p.lon + c));
   const int tz = p.tz_idx ? (int)__ldg(p.tz_idx + c) : 0;
 
@@ -500,6 +531,32 @@ __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f3
 #undef TFG_PUT
       }
     }
+    if constexpr (OBJ) {
+      // the step's value of the chosen BMI output against the observation of the cell's column; a non-finite
+      // observation is "not observed" (the cell's own value may be NaN: a poisoned cell is scored, and its sums say so)
+      if (t >= p.obj_t_lo && t < p.obj_t_hi) {   // warp-uniform
+        const int64_t col = p.obj_col ? (int64_t)__ldg(p.obj_col + c) : c;
+        const double ob = __ldg(p.obj_obs + (int64_t)(t - p.obj_t_lo) * p.obj_ncols + col);
+        if (((unsigned)__double2hiint(ob) & 0x7ff00000u) != 0x7ff00000u) {
+          raw v;
+          switch (p.obj_quantity) {   // a kernel parameter: warp-uniform
+            case TFG_REC_H_SNOW: v = st.h_snow; break;
+            case TFG_REC_H_SWE: v = st.h_swe; break;
+            case TFG_REC_SM: v = o.SM; break;
+            case TFG_REC_H_ICE: v = st.h_ice; break;
+            case TFG_REC_H_IWE: v = st.h_iwe; break;
+            case TFG_REC_IM: v = o.IM; break;
+            case TFG_REC_M_TOTAL: v = o.M_total; break;
+            default: v = o.RH; break;
+          }
+          const double sv = (double)v, d = __dsub_rn(sv, ob);   // float32: widened exactly
+          osum.set(0, __dadd_rn(osum.get(0), sv));
+          osum.set(1, __dadd_rn(osum.get(1), __dmul_rn(sv, sv)));
+          osum.set(2, __dadd_rn(osum.get(2), __dmul_rn(sv, ob)));
+          osum.set(3, __dadd_rn(osum.get(3), __dmul_rn(d, d)));
+        }
+      }
+    }
     if constexpr (AGG) {
       if (have_agg) {
         // area-weighted basin sums (np.sum sites :567-568,:1486-1494 and the driver's `* da_m2`):
@@ -568,6 +625,10 @@ __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f3
       p.vol_P[c] = s.get(kSVolP); p.vol_PR[c] = s.get(kSVolPR); p.vol_PS[c] = s.get(kSVolPS);
       p.vol_SM[c] = s.get(kSVolSM); p.vol_IM[c] = s.get(kSVolIM); p.P_max[c] = s.get(kSPmax);
     }
+    if constexpr (OBJ) {
+#pragma unroll
+      for (int i = 0; i < TFG_N_OBJ; ++i) p.obj_acc[(int64_t)i * N + c] = osum.get(i);
+    }
   }
 }
 
@@ -613,6 +674,20 @@ cudaError_t launch_run_as(const RunParams<typename P::raw>& p, bool rec, bool ag
                    ((reinterpret_cast<uintptr_t>(p.forcing) & 15) == 0) &&
                    ((p.n_cells * sizeof(typename P::raw)) % 16 == 0);
   const size_t dyn = P::lean ? fm::kTabDoubles * sizeof(double) : 0;
+  if (p.obj_acc != nullptr) {
+    // objective bound: two kernel shapes only, both of which test basin_agg and vol_P at run time (register prefetch,
+    // like PAR); the recording one for launches that record
+    if constexpr (!P::f32) {
+      if (p.col_terms != nullptr) {
+        if (rec) run_kernel<P, true, true, true, false, true, PAR, true><<<grid, kBlock, dyn, stream>>>(p);
+        else run_kernel<P, false, true, true, false, true, PAR, true><<<grid, kBlock, dyn, stream>>>(p);
+        return cudaGetLastError();
+      }
+    }
+    if (rec) run_kernel<P, true, true, true, false, false, PAR, true><<<grid, kBlock, dyn, stream>>>(p);
+    else run_kernel<P, false, true, true, false, false, PAR, true><<<grid, kBlock, dyn, stream>>>(p);
+    return cudaGetLastError();
+  }
   if constexpr (!P::f32) {
     if (p.col_terms != nullptr) {  // column terms bound (forcing map): the kernel reads them instead of the forcing block
       if (rec) run_kernel<P, true, true, true, false, true, PAR><<<grid, kBlock, dyn, stream>>>(p);
@@ -639,7 +714,8 @@ cudaError_t launch_run_as(const RunParams<typename P::raw>& p, bool rec, bool ag
   return cudaGetLastError();
 }
 
-// per-cell surface parameters bound (tfg_bind_cell_params): the PAR instantiations, chosen from the input
+// per-cell surface parameters bound (tfg_bind_cell_params): the PAR instantiations, chosen from the input; an objective
+// bound (p.obj_acc): the OBJ instantiations (launch_run_as)
 template <class P>
 cudaError_t launch_run(const RunParams<typename P::raw>& p, bool rec, bool agg, bool vol, cudaStream_t stream) {
   return p.cell_par != nullptr ? launch_run_as<P, true>(p, rec, agg, vol, stream) : launch_run_as<P, false>(p, rec, agg, vol, stream);

@@ -120,6 +120,7 @@ class MeltEngine:
             self.tz_idx = None if tz_idx is None else torch.as_tensor(
                 np.ascontiguousarray(tz_idx, dtype=np.uint8)).to(self.device)
             self._bind_static()
+            self.objective = None
             self.cell_params = None
             if cell_params is not None:
                 self.set_cell_params(cell_params)
@@ -181,6 +182,96 @@ class MeltEngine:
             # the library derives its own copy on the current stream and waits for its range check
             _lib.check(self.lib.tfg_bind_cell_params(self.ctx, C.byref(p), self.stream_ptr), "tfg_bind_cell_params")
         self.cell_params = bound
+
+    # ---- objective: scores of every cell against observations, accumulated inside the melt kernel ----------------
+    def set_objective(self, quantity: Optional[str], obs=None, obs_step0: int = 0, obs_index=None) -> None:
+        """Score one BMI output of every cell against observations in every later ``run`` (``tfg_bind_objective``).
+
+        ``quantity`` is one of the eight BMI outputs (``REC_NAMES[:8]``: ``h_snow, h_swe, SM, h_ice, h_iwe, IM,
+        M_total, RH``); ``None`` unbinds.  ``obs`` is ``[T_obs, n_obs_cols]`` (host or device), row ``j`` the observation
+        of absolute step ``obs_step0 + j``; NaN = not observed (daily values of an hourly run, a spin-up period).
+        Cell ``i`` reads column ``obs_index[i]``; the default is the forcing map when one is bound (one column per
+        catchment), else the identity (``n_obs_cols == N``).  The sums start at zero; ``scores()`` reads them and
+        ``reset_objective()`` zeroes them (after ``load_state_dict`` in a calibration loop)."""
+        if quantity is None:
+            _lib.check(self.lib.tfg_bind_objective(self.ctx, None, self.stream_ptr), "tfg_bind_objective")
+            self.objective = None
+            return
+        q = _lib.REC_BIT.get(quantity, -1)
+        if not 0 <= q < 8:
+            raise ValueError(f"quantity must be one of the eight BMI outputs {_lib.REC_NAMES[:8]}, got {quantity!r}")
+        o = (obs if torch.is_tensor(obs) else torch.as_tensor(np.asarray(obs, dtype=np.float64)))
+        if o.dim() != 2 or o.shape[0] < 1 or o.shape[1] < 1:
+            raise ValueError(f"obs must be [T_obs, n_obs_cols] with both > 0, got shape {tuple(o.shape)}")
+        o = o.to(self.device, torch.float64).contiguous()
+        if obs_index is None:
+            obs_index = self.forcing_index
+        idx = None
+        if obs_index is not None:
+            idx = (obs_index if torch.is_tensor(obs_index) else torch.as_tensor(np.ascontiguousarray(obs_index)))
+            idx = idx.to(self.device, torch.int32).contiguous().reshape(-1)
+            if idx.numel() != self.N:
+                raise ValueError(f"obs_index must have one entry per cell ({self.N}), got {idx.numel()}")
+        elif o.shape[1] != self.N:
+            raise ValueError(f"obs must have one column per cell ({self.N}) without obs_index, got {o.shape[1]}")
+        acc = torch.zeros(_lib.N_OBJ, self.N, dtype=torch.float64, device=self.device)
+        b = _lib.Objective(quantity=q, obs=o.data_ptr(), obs_step0=int(obs_step0), n_obs_steps=o.shape[0],
+                           n_obs_cols=o.shape[1], obs_col=idx.data_ptr() if idx is not None else None, acc=acc.data_ptr())
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.tfg_bind_objective(self.ctx, C.byref(b), self.stream_ptr), "tfg_bind_objective")
+        self.objective = {"quantity": quantity, "obs": o, "obs_step0": int(obs_step0), "obs_index": idx, "acc": acc,
+                          "row_counts": np.zeros(o.shape[0], dtype=np.int64), "moments": None}
+
+    def reset_objective(self) -> None:
+        """Zero the objective's sums and the count of scored observation rows (e.g. after ``load_state_dict``)."""
+        ob = self._objective_or_raise()
+        ob["acc"].zero_()
+        ob["row_counts"][:] = 0
+        ob["moments"] = None
+
+    def objective_sums(self):
+        """The kernel's four ``[N]`` float64 sums ``(S_s, S_ss, S_so, S_ee)`` (views of the accumulators)."""
+        acc = self._objective_or_raise()["acc"]
+        return acc[0], acc[1], acc[2], acc[3]
+
+    def objective_moments(self):
+        """``(n, S_o, S_oo)`` of the observations each cell was scored against, ``[N]`` float64 each.
+
+        Formed from ``obs`` and the count of launches that scored each row: rows in time order, each added as often as
+        it was scored, with the kernel's operations -- so after one pass over the window they are the bits the kernel
+        would form from the observations themselves."""
+        from .objective import accumulate_step
+
+        ob = self._objective_or_raise()
+        if ob["moments"] is None:
+            mom = torch.zeros(3, ob["obs"].shape[1], dtype=torch.float64, device=self.device)
+            for j in np.nonzero(ob["row_counts"])[0]:
+                for _ in range(int(ob["row_counts"][j])):
+                    accumulate_step(None, mom, None, ob["obs"][j])
+            ob["moments"] = mom
+        m = ob["moments"] if ob["obs_index"] is None else ob["moments"][:, ob["obs_index"].to(torch.int64)]
+        return m[0], m[1], m[2]
+
+    def scores(self) -> dict:
+        """``{n, nse, kge, r, alpha, beta, rmse, bias}``: ``[N]`` float64 device tensors (``objective.skill_scores``).
+        Observation rows scored twice (a rewind without ``reset_objective``) count twice on both sides."""
+        from .objective import skill_scores
+
+        return skill_scores(self.objective_sums(), self.objective_moments())
+
+    def _objective_or_raise(self) -> dict:
+        if getattr(self, "objective", None) is None:
+            raise RuntimeError("no objective bound (set_objective)")
+        return self.objective
+
+    def _count_scored_rows(self, step0: int, n_steps: int) -> None:
+        """Count the observation rows a run of [step0, step0 + n_steps) scored (for objective_moments)."""
+        ob = self.objective
+        w0 = ob["obs_step0"]
+        lo, hi = max(step0, w0), min(step0 + n_steps, w0 + ob["obs"].shape[0])
+        if lo < hi:
+            ob["row_counts"][lo - w0:hi - w0] += 1
+            ob["moments"] = None
 
     def _init_state(self, init):
         """Initial state of reference ``initialize()`` (``:350-395``): depths from the config, albedo 0.3,
@@ -286,6 +377,8 @@ class MeltEngine:
                 self.ctx, forcing.data_ptr(), self.step_index, T, rec_t.data_ptr() if rec_t is not None else None,
                 mask, basin_agg.data_ptr() if basin_agg is not None else None, self.n_basin, self.stream_ptr),
                 "tfg_run")
+            if self.objective is not None:
+                self._count_scored_rows(self.step_index, T)
         self.step_index += T
         return {k: rec_t[:, i] for i, k in enumerate(names)} if rec_t is not None else {}
 

@@ -237,6 +237,39 @@ class ShardedMeltEngine:
         agg.reduce()
         return rec, agg.buffer
 
+    def set_objective(self, quantity, obs=None, obs_step0: int = 0, obs_index=None):
+        """``MeltEngine.set_objective`` on every rank.  ``obs`` is the whole ``[T_obs, n_obs_cols]`` block (every rank
+        holds it); ``obs_index`` is a GLOBAL per-cell array, sliced here like ``cell_params``.  Without it each cell reads
+        its forcing column when a forcing map is bound, else its own global column (``n_obs_cols == n_total``)."""
+        lo, hi = self.bounds
+        if quantity is not None and obs_index is None and self.engine.forcing_index is None:
+            obs_index = np.arange(self.n_total, dtype=np.int32)
+        if obs_index is not None:
+            obs_index = obs_index[lo:hi]
+        self.engine.set_objective(quantity, obs, obs_step0=obs_step0, obs_index=obs_index)
+
+    def scores(self, gather: bool = True) -> dict:
+        """The local shard's ``MeltEngine.scores()``; with ``gather`` (a collective: call on all ranks) the scores of all
+        ``n_total`` cells on every rank, so that each rank can pick the best candidate per catchment."""
+        import torch
+
+        local = self.engine.scores()
+        if not gather or self.world == 1:
+            return local
+        import torch.distributed as dist
+
+        names = list(local)
+        block = torch.stack([local[k] for k in names])                      # [K, n_local]
+        if dist.get_backend(self.group) == "gloo":
+            block = block.cpu()
+        sizes = [b - a for a, b in (shard_bounds(self.n_total, self.world, r) for r in range(self.world))]
+        pad = torch.full((len(names), max(sizes)), float("nan"), dtype=torch.float64, device=block.device)
+        pad[:, :block.shape[1]] = block
+        parts = [torch.empty_like(pad) for _ in range(self.world)]
+        dist.all_gather(parts, pad, group=self.group)
+        full = torch.cat([p[:, :n] for p, n in zip(parts, sizes)], dim=1).to(local[names[0]].device)
+        return {k: full[i] for i, k in enumerate(names)}
+
     def basin_area(self):
         """Global per-basin area ``sum(da_m2)`` (all ranks)."""
         return self.aggregates(1).basin_area(self.engine.static["da_m2"], self.engine.basin_id)
