@@ -129,13 +129,17 @@ TFG_API int tfg_mode(const tfg_ctx* ctx);
  * (4 stages) instead of per-thread prefetching loads; results are bit-identical either way */
 #define TFG_OPT_TMA_STAGING 1
 /* TFG_OPT_EXACT_AGG: order-independent basin aggregates.  value = 0 switches it off; otherwise
- * value = 1<<24 | (E2+128)<<16 | (E1+128)<<8 | (E0+128), E_q the binary exponent that bounds a 32-cell partial sum
- * of aggregate q (|partial| < 2^E_q).  tfg_run then reads `basin_agg` as int64 [n_steps][n_basin][TFG_N_AGG][2]
- * followed by ONE trailing int64 counter: every contribution is split into two fixed-point words
- * (value = hi * 2^(E_q-40) + lo * 2^(E_q-82)) that are added with integer atomics, so the sums do not depend on the
- * order of the atomics, on the launch geometry or on how cells are sharded over GPUs (32-cell aligned shards), and
- * an integer all-reduce of the accumulators is exact.  Contributions that are not finite or exceed 2^E_q are left
- * out and counted in the trailing word.                                                                        */
+ * value = L<<32 | 1<<24 | (E2+128)<<16 | (E1+128)<<8 | (E0+128), E_q the binary exponent that bounds a 32-cell partial
+ * sum of aggregate q (|partial| < 2^E_q), L in [1, 62] the fraction bits of the low word (L = 0 means 42; bits 40-63
+ * must be 0).  tfg_run then reads `basin_agg` as int64 [n_steps][n_basin][TFG_N_AGG][2] followed by ONE trailing
+ * int64 counter: every contribution v is split into two fixed-point words, hi = trunc(v * 2^(40-E_q)) and
+ * lo = trunc(frac(v * 2^(40-E_q)) * 2^L) (value = hi * 2^(E_q-40) + lo * 2^(E_q-40-L)), that are added with integer
+ * atomics, so the sums do not depend on the order of the atomics, on the launch geometry or on how cells are sharded
+ * over GPUs (32-cell aligned shards), and an integer all-reduce of the accumulators is exact.  Contributions that are
+ * not finite or reach 2^E_q are left out and counted in the trailing word.
+ * Headroom: with C contributions to one (step, basin, aggregate) the low word stays below C * 2^L and the high word
+ * below C * 2^40; the caller picks L <= 62 - ceil(log2 C) (a warp of 32 cells inside one basin is one contribution,
+ * every cell of a warp that straddles basins is one).  Words that leave the int64 range wrap without notice. */
 #define TFG_OPT_EXACT_AGG 2
 /* TFG_OPT_COLUMN_TERMS (default 1; TFG_F64_FAST and TFG_F64_STRICT contexts with a forcing map of at most n_cells / 8 columns): the part of
  * update() that reads nothing but the forcings (vapour pressures, relative humidity, dew point, precipitable water,

@@ -218,7 +218,9 @@ def test_exact_basin_aggregates_are_order_and_sharding_independent(cuda_device):
         st = {k: v[lo:hi] for k, v in statics.items()}
         eng = MeltEngine(st, default_constants(), "2013040100", zones=[-8.0], mode="f64_fast", basin_id=basin_id[lo:hi],
                          n_basin=NB, horizon_steps=T + 1)
-        agg = BasinAggregates(T, NB, device=cuda_device, exponents=exps or eng.agg_exponents())
+        if exps is not None:
+            eng.set_agg_exponents(exps)          # the shards scale with the whole grid's exponents, as ranks do
+        agg = BasinAggregates(T, NB, device=cuda_device, exponents=eng.agg_exponents())
         rec = eng.run(f[:, :, lo:hi].contiguous(), record=("M_total", "h_swe", "h_iwe"), basin_agg=agg.zero())
         torch.cuda.synchronize()
         out = (agg, {k: v.cpu().numpy() for k, v in rec.items()}, eng.agg_exponents())

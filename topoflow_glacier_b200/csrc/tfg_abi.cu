@@ -204,6 +204,8 @@ tfg::RunParams<raw> make_params(const tfg_ctx* x, const void* forcing, int64_t s
   p.agg_bad = agg_bad;
   for (int q = 0; q < TFG_N_AGG; ++q)  // 2^(40 - E_q): scales a partial sum into the hi fixed-point word
     p.agg_up[q] = ldexp(1.0, 40 - ((int)((x->exact_agg >> (8 * q)) & 0xff) - 128));
+  const int lo_bits = (int)((x->exact_agg >> 32) & 0xff);  // L, the low word's fraction bits; 0 = 42
+  p.agg_lo = ldexp(1.0, lo_bits ? lo_bits : 42);
   p.n_basin = n_basin;
   p.k = derive<raw>(x->c);
   p.cell_par = x->have_cell_par ? static_cast<const raw*>(x->cell_par) : nullptr;
@@ -421,7 +423,12 @@ size_t tfg_elem_size(const tfg_ctx* x) { return (x && x->mode == TFG_F32) ? 4 : 
 int tfg_set_option(tfg_ctx* x, int option, int64_t value) {
   if (!x) return fail("tfg_set_option: NULL context");
   if (option == TFG_OPT_TMA_STAGING) { x->use_tma = value != 0; return 0; }
-  if (option == TFG_OPT_EXACT_AGG) { x->exact_agg = value; return 0; }
+  if (option == TFG_OPT_EXACT_AGG) {
+    if (value != 0 && (((value >> 32) & 0xff) > 62 || (value >> 40) != 0))
+      return fail("tfg_set_option: TFG_OPT_EXACT_AGG: low-word bits L (bits 32-39) must be at most 62, bits 40-63 zero");
+    x->exact_agg = value;
+    return 0;
+  }
   if (option == TFG_OPT_COLUMN_TERMS) { x->column_terms = value != 0; return 0; }
   return fail("tfg_set_option: unknown option");
 }

@@ -659,7 +659,7 @@ __global__ void __launch_bounds__(kLeanBlock, TFG_LEAN_MIN_BLOCKS) run_kernel_le
           kk += __shfl_xor_sync(full, kk, 2);
           kk += __shfl_xor_sync(full, kk, 1);
           if ((lane & 7) == 0 && lane < 24) {
-            if (p.agg_exact) agg_add_exact(acc + 2 * (lane >> 3), kk, p.agg_up[lane >> 3], p.agg_bad);
+            if (p.agg_exact) agg_add_exact(acc + 2 * (lane >> 3), kk, p.agg_up[lane >> 3], p.agg_lo, p.agg_bad);
             else atomicAdd(dst + (lane >> 3), kk);
           }
         } else {
@@ -669,8 +669,8 @@ __global__ void __launch_bounds__(kLeanBlock, TFG_LEAN_MIN_BLOCKS) run_kernel_le
             double* dst = static_cast<double*>(p.basin_agg) + entry;
             long long* acc = static_cast<long long*>(p.basin_agg) + 2 * entry;
             if (p.agg_exact) {
-              agg_add_exact(acc + 0, v0[w], p.agg_up[0], p.agg_bad); agg_add_exact(acc + 2, v1[w], p.agg_up[1], p.agg_bad);
-              agg_add_exact(acc + 4, v2[w], p.agg_up[2], p.agg_bad);
+              agg_add_exact(acc + 0, v0[w], p.agg_up[0], p.agg_lo, p.agg_bad); agg_add_exact(acc + 2, v1[w], p.agg_up[1], p.agg_lo, p.agg_bad);
+              agg_add_exact(acc + 4, v2[w], p.agg_up[2], p.agg_lo, p.agg_bad);
             } else {
               atomicAdd(dst + 0, v0[w]); atomicAdd(dst + 1, v1[w]); atomicAdd(dst + 2, v2[w]);
             }

@@ -87,6 +87,8 @@ struct RunParams {
   const int32_t* obj_col;      // [n_cells] or nullptr (column = cell)
   int64_t obj_ncols;
   int32_t obj_t_lo, obj_t_hi, obj_quantity;
+  double agg_lo;               // 2^L: fraction bits of the low word of exact aggregates (with agg_up; here, behind the
+                               // members above, so that the kernels without aggregates keep their parameter offsets)
 };
 
 template <class raw> __device__ __forceinline__ raw ld_stream(const raw* p) { return __ldcs(p); }
@@ -175,16 +177,17 @@ __device__ __noinline__ Num<P> window_sum_exact(const typename P::raw* ring, int
   return res;
 }
 
-// One contribution to an exact basin aggregate: v * up = a + r with a = trunc (|a| < 2^40), b = trunc(r * 2^42);
-// both words are added with integer atomics (associative, hence order-independent).
-__device__ __forceinline__ void agg_add_exact(long long* acc, double v, double up, long long* bad) {
+// One contribution to an exact basin aggregate: v * up = a + r with a = trunc (|a| < 2^40), b = trunc(r * lo), lo = 2^L;
+// both words are added with integer atomics (associative, hence order-independent).  The host chooses L so that the
+// low word of C contributions, |sum| < C * 2^L, stays below 2^63 (MeltEngine.agg_exponents).
+__device__ __forceinline__ void agg_add_exact(long long* acc, double v, double up, double lo, long long* bad) {
   const double s = v * up;  // a power-of-two scaling: exact
   if (!(fabs(s) < 1099511627776.0)) {  // also catches NaN
     if (bad) atomicAdd(reinterpret_cast<unsigned long long*>(bad), 1ull);
     return;
   }
   const long long a = __double2ll_rz(s);
-  const long long b = __double2ll_rz((s - (double)a) * 4398046511104.0);
+  const long long b = __double2ll_rz((s - (double)a) * lo);
   if (a) atomicAdd(reinterpret_cast<unsigned long long*>(acc), (unsigned long long)a);
   if (b) atomicAdd(reinterpret_cast<unsigned long long*>(acc) + 1, (unsigned long long)b);
 }
@@ -585,13 +588,14 @@ __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f3
           k += __shfl_xor_sync(full, k, 2);
           k += __shfl_xor_sync(full, k, 1);
           if ((lane & 7) == 0 && lane < 24) {
-            if (p.agg_exact) agg_add_exact(acc + 2 * (lane >> 3), k, p.agg_up[lane >> 3], p.agg_bad);
+            if (p.agg_exact) agg_add_exact(acc + 2 * (lane >> 3), k, p.agg_up[lane >> 3], p.agg_lo, p.agg_bad);
             else atomicAdd(dst + (lane >> 3), k);
           }
         } else if (active) {
           if (p.agg_exact) {
-            agg_add_exact(acc + 0, v0, p.agg_up[0], p.agg_bad); agg_add_exact(acc + 2, v1, p.agg_up[1], p.agg_bad);
-            agg_add_exact(acc + 4, v2, p.agg_up[2], p.agg_bad);
+            agg_add_exact(acc + 0, v0, p.agg_up[0], p.agg_lo, p.agg_bad);
+            agg_add_exact(acc + 2, v1, p.agg_up[1], p.agg_lo, p.agg_bad);
+            agg_add_exact(acc + 4, v2, p.agg_up[2], p.agg_lo, p.agg_bad);
           } else {
             atomicAdd(dst + 0, v0); atomicAdd(dst + 1, v1); atomicAdd(dst + 2, v2);
           }

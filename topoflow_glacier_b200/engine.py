@@ -416,27 +416,55 @@ class MeltEngine:
 
     # ---- order-independent basin aggregates (TFG_OPT_EXACT_AGG, include/tfglacier.h) ---------------------------
     def agg_exponents(self):
-        """Binary exponents E_q with |32-cell partial of aggregate q| < 2^E_q for physically possible values:
-        M_total < 2^-8 m/s (10 m/h of rain is 2.8e-3), water-equivalent depths < 2^17 m."""
+        """Scaling of the exact aggregates, ``(E0, E1, E2, L)`` (``sharding.agg_scaling``): binary exponents E_q with
+        |32-cell partial of aggregate q| < 2^E_q for physically possible values -- M_total < 2^-8 m/s (10 m/h of rain
+        is 2.8e-3), water-equivalent depths < 2^17 m -- and the fraction bits L of the low word, chosen from the count
+        of contributions to one basin so that neither word can leave the int64 range.  Under ``torch.distributed``
+        the largest cell area and the per-basin counts are agreed over all ranks (collective: call on all ranks).
+        ``set_agg_exponents`` pins other values instead."""
         if self._agg_exp is None:
-            da_max_t = self.static["da_m2"].max().to(torch.float64)
+            self._agg_exp = self._agg_scaling(reduce=True)
+        return self._agg_exp
+
+    def _agg_scaling(self, reduce: bool):
+        from .sharding import agg_contributions, agg_scaling
+
+        da_max_t = self.static["da_m2"].max().to(torch.float64)
+        counts = torch.stack(agg_contributions(self.basin_id, self.n_basin))
+        if reduce:
             try:  # every rank must scale with the SAME exponents, or the integer all-reduce adds apples and pears
                 import torch.distributed as dist
 
                 if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
                     dist.all_reduce(da_max_t, op=dist.ReduceOp.MAX)   # collective: call on all ranks
+                    dist.all_reduce(counts, op=dist.ReduceOp.SUM)
             except ImportError:
                 pass
-            da_max = float(da_max_t.item())
-            e_da = int(np.ceil(np.log2(max(da_max, 1e-30) * 32.0)))
-            self._agg_exp = (e_da - 8, e_da + 17, e_da + 17)
-        return self._agg_exp
+        counts = counts.cpu().numpy()
+        return agg_scaling(float(da_max_t.item()), counts[0], counts[1])
+
+    def set_agg_exponents(self, exps) -> None:
+        """Scale this engine's exact aggregates with ``exps`` (``(E0, E1, E2)`` or ``(E0, E1, E2, L)``; 3 values mean
+        L = 42) instead of its own ``agg_exponents()``.  For engines in one process whose words are added together: all
+        must scale alike, e.g. with the exponents of an engine over all their cells.  Exponents smaller than this
+        engine's cells need, or an L larger than its own basin counts allow, are refused (ValueError); the caller
+        answers for the sum of the counts over the engines it adds."""
+        e = tuple(int(x) for x in exps)
+        if len(e) == 3:
+            e += (42,)
+        if len(e) != 4:
+            raise ValueError(f"exponents must be (E0, E1, E2) or (E0, E1, E2, L), got {exps!r}")
+        need = self._agg_scaling(reduce=False)
+        if any(e[q] < need[q] for q in range(3)) or not 1 <= e[3] <= need[3]:
+            raise ValueError(f"exact aggregates of this engine need exponents >= {need[:3]} and 1 <= L <= {need[3]}, "
+                             f"got {e}")
+        self._agg_exp = e
 
     def exact_agg_option(self) -> int:
         e = self.agg_exponents()
-        if not all(-128 <= x < 128 for x in e):
+        if not all(-128 <= x < 128 for x in e[:3]):
             raise ValueError("cell areas out of range for exact aggregates")
-        return (1 << 24) | ((e[2] + 128) << 16) | ((e[1] + 128) << 8) | (e[0] + 128)
+        return (e[3] << 32) | (1 << 24) | ((e[2] + 128) << 16) | ((e[1] + 128) << 8) | (e[0] + 128)
 
     def step(self, record: Optional[Iterable[str]] = None):
         """One literal ``update()`` from the current input block."""

@@ -14,7 +14,8 @@ from typing import Optional, Tuple
 
 import numpy as np
 
-__all__ = ["shard_bounds", "shard_sizes", "BasinAggregates", "basin_sums_host", "dist_info", "ShardedMeltEngine"]
+__all__ = ["shard_bounds", "shard_sizes", "BasinAggregates", "agg_contributions", "agg_scaling", "basin_sums_host", "dist_info",
+           "ShardedMeltEngine"]
 
 AGG_NAMES = ("runoff_m3s", "swe_m3", "iwe_m3")  # sum(M_total*da_m2), sum(h_swe*da_m2), sum(h_iwe*da_m2)
 
@@ -63,6 +64,49 @@ def dist_info() -> Tuple[int, int]:
     return 0, 1
 
 
+def agg_contributions(basin_id, n_basin: int):
+    """Contributions of one timestep to each basin's exact aggregate: ``(cells, warps)``, int64 ``[n_basin]`` tensors.
+
+    The kernel adds one partial sum per warp of 32 consecutive cells that lie in one basin (``warps``) and one value
+    per cell of a warp that straddles basins (``cells``); lanes past the last cell carry the last cell's basin.  Counts
+    are exact, so they add over 128-cell aligned shards.  ``basin_id`` is a torch tensor (any device) or None."""
+    import torch
+
+    if basin_id is None or basin_id.numel() == 0:
+        z = torch.zeros(max(int(n_basin), 0), dtype=torch.int64)
+        return z, z.clone()
+    b = basin_id.reshape(-1).to(torch.int64)
+    n = b.numel()
+    if int(b.min()) < 0 or int(b.max()) >= n_basin:
+        raise ValueError(f"basin ids must lie in [0, n_basin = {n_basin})")
+    w = torch.cat([b, b[-1:].expand((-n) % 32)]).view(-1, 32)
+    uniform = (w == w[:, :1]).all(dim=1)
+    warps = torch.bincount(w[uniform, 0], minlength=n_basin)
+    real = (torch.arange(w.numel(), device=b.device) < n).view(-1, 32)
+    cells = torch.bincount(w[~uniform][real[~uniform]], minlength=n_basin)
+    return cells, warps
+
+
+def agg_scaling(da_max: float, cells, warps):
+    """``(E0, E1, E2, L)`` of exact aggregates over cells of at most ``da_max`` m2 and the per-basin contribution counts
+    ``cells``, ``warps`` of ``agg_contributions`` (summed over all ranks whose words are added).
+
+    E_q bounds a 32-cell partial sum: |partial| < 2^E_q for M_total < 2^-8 m/s and depths < 2^17 m.  A contribution
+    adds less than 2^L to the low word, so with C = max over basins of (cells + warps) contributions the low word stays
+    below C * 2^L <= 2^62 for L = min(42, 62 - ceil(log2 C)).  The high word gains less than 2^35 per cell (one cell is
+    at most 1/32 of the bound of a partial) and less than 2^40 per warp partial; a layout that could take it to 2^63
+    has no safe scaling and raises ValueError, as the words would otherwise wrap without notice."""
+    e_da = int(np.ceil(np.log2(max(float(da_max), 1e-30) * 32.0)))
+    per_basin = [int(c) + int(w) for c, w in zip(cells, warps)]
+    n_max = max(per_basin, default=1) or 1
+    lo_bits = min(42, 62 - (n_max - 1).bit_length())
+    hi_max = max((int(c) * 2**35 + int(w) * 2**40 for c, w in zip(cells, warps)), default=0)
+    if lo_bits < 1 or hi_max >= 2**63:
+        raise ValueError(f"exact aggregates: {n_max} contributions to one basin and step could overflow the int64 "
+                         "words; split the basin or use the floating-point aggregates")
+    return e_da - 8, e_da + 17, e_da + 17, lo_bits
+
+
 def basin_sums_host(values: np.ndarray, da_m2: np.ndarray, basin_id: np.ndarray, n_basin: int) -> np.ndarray:
     """Host statement of one aggregate: ``out[b] = sum(values[i] * da_m2[i] for basin_id[i] == b)``."""
     return np.bincount(basin_id, weights=np.asarray(values, dtype=np.float64) * da_m2, minlength=n_basin)
@@ -75,13 +119,14 @@ class BasinAggregates:
     floating-point atomics; ``reduce`` makes it global (in place) with one ``all_reduce(SUM)``.  Reproducible to
     rounding (~1e-15), not bit for bit: the order of the atomics is not fixed.
 
-    ``exponents=(E0, E1, E2)`` (``MeltEngine.agg_exponents()``, which agrees them across ranks with one
-    ``all_reduce(MAX)`` -- every rank must scale with the same exponents) selects ORDER-INDEPENDENT sums instead: the kernel
-    splits every contribution into two fixed-point int64 words and adds them with integer atomics
-    (``TFG_OPT_EXACT_AGG``); ``accumulator`` is that int64 tensor (pass it to ``MeltEngine.run(basin_agg=...)``),
-    ``reduce`` all-reduces the integers -- exactly -- and decodes them into ``buffer``.  The result is bit-identical
-    for any GPU count (shards are 128-cell aligned), launch split or scheduling order.  Works on CUDA tensors with
-    NCCL and on CPU tensors with gloo.
+    ``exponents=(E0, E1, E2, L)`` (``MeltEngine.agg_exponents()``, which agrees them across ranks with all-reduces --
+    every rank must scale with the same exponents; a 3-tuple means L = 42) selects ORDER-INDEPENDENT sums instead: the
+    kernel splits every contribution into two fixed-point int64 words and adds them with integer atomics
+    (``TFG_OPT_EXACT_AGG``); ``accumulator`` is that int64 tensor (pass it to ``MeltEngine.run(basin_agg=...)`` of an
+    engine that scales with the same exponents), ``reduce`` all-reduces the integers -- exactly -- and decodes them into
+    ``buffer``.  The result is bit-identical for any GPU count (shards are 128-cell aligned), launch split or
+    scheduling order, and lies within C * 2^(E-40-L) of the exact sum of the contributions (C of them, each truncated
+    once) plus the rounding of the decode.  Works on CUDA tensors with NCCL and on CPU tensors with gloo.
     """
 
     def __init__(self, chunk_steps: int, n_basin: int, device=None, group=None, exponents=None):
@@ -95,9 +140,13 @@ class BasinAggregates:
         self.exponents = None if exponents is None else tuple(int(e) for e in exponents)
         self.accumulator = None
         if self.exponents is not None:
+            if len(self.exponents) == 3:
+                self.exponents += (42,)
+            if len(self.exponents) != 4:
+                raise ValueError(f"exponents must be (E0, E1, E2) or (E0, E1, E2, L), got {exponents!r}")
             self.accumulator = torch.zeros(self.chunk_steps * self.n_basin * 3 * 2 + 1, dtype=torch.int64, device=device)
-            e = torch.tensor(self.exponents, dtype=torch.float64, device=device)
-            self._scale_hi, self._scale_lo = torch.exp2(e - 40.0), torch.exp2(e - 82.0)
+            e = torch.tensor(self.exponents[:3], dtype=torch.float64, device=device)
+            self._scale_hi, self._scale_lo = torch.exp2(e - 40.0), torch.exp2(e - 40.0 - self.exponents[3])
 
     @property
     def target(self):
@@ -116,7 +165,7 @@ class BasinAggregates:
         return self.target
 
     def decode(self):
-        """int64 {hi, lo} words -> float64 ``buffer`` (value = hi * 2^(E-40) + lo * 2^(E-82)); a pure function of
+        """int64 {hi, lo} words -> float64 ``buffer`` (value = hi * 2^(E-40) + lo * 2^(E-40-L)); a pure function of
         the integer sums, hence as reproducible as they are."""
         w = self.accumulator[:-1].view(self.chunk_steps, self.n_basin, 3, 2).to(self.torch.float64)
         self.torch.add(w[..., 0] * self._scale_hi, w[..., 1] * self._scale_lo, out=self.buffer)
