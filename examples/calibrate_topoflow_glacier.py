@@ -1,7 +1,7 @@
 """Random-search calibration of the five surface parameters over the shipped catchments, scored on the device.
 
     python examples/calibrate_topoflow_glacier.py [--sets 256] [--mode f64|f64_fast|f32] [--quantity M_total] [--daily]
-                                                  [--obs FILE.csv] [--write-obs FILE.csv] [--seed 0]
+                                                  [--obs FILE.csv] [--write-obs FILE.csv] [--seed 0] [--forcing-params]
 
 Every catchment of ``config/`` (``cat-*.yaml`` except the ``-const`` variant) gets ``--sets`` candidate parameter sets,
 drawn uniformly from the schema's ranges of ``dust_atten, canopy_factor, cloud_factor, z0_air, em_surf``.  All
@@ -20,6 +20,10 @@ day, a once-a-day reading); the other rows are NaN.
 ``--obs FILE.csv`` reads real observations instead: a ``Time`` column (``YYYY-MM-DD HH:MM``) plus one column per
 catchment, named after its yaml (``cat-3062784`` ...); a blank cell is a missing observation.
 ``--write-obs`` writes the observations in that format.
+``--forcing-params`` also draws the two forcing parameters that matter most in glacier mass-balance calibration, a
+temperature bias ``T_air_offset`` in [-3, 3] K and a precipitation factor ``P_multiplier`` in [0.5, 2]
+(``MeltEngine(forcing_adjust=...)``): each candidate then adjusts the catchment's shared series inside the melt kernel.
+The twin experiment's truth draws them from the same ranges.
 
 ``run()`` returns the best candidate per catchment and all scores, like ``run_topoflow_glacier.run``.
 """
@@ -53,9 +57,16 @@ def catchments():
     return out
 
 
-def draw(rng, n):
-    """n parameter sets, uniform in the schema's ranges: {key: [n]}."""
-    return {k: rng.uniform(lo, hi, n) for k, (lo, hi) in CELL_PARAM_RANGES.items()}
+# ranges of the forcing parameters drawn with --forcing-params (narrower than the engine accepts)
+FORCING_DRAW = {"T_air_offset": (-3.0, 3.0), "P_multiplier": (0.5, 2.0)}
+
+
+def draw(rng, n, forcing_params=False):
+    """n parameter sets, uniform in the schema's ranges (and FORCING_DRAW's with ``forcing_params``): {key: [n]}."""
+    out = {k: rng.uniform(lo, hi, n) for k, (lo, hi) in CELL_PARAM_RANGES.items()}
+    if forcing_params:
+        out.update({k: rng.uniform(lo, hi, n) for k, (lo, hi) in FORCING_DRAW.items()})
+    return out
 
 
 def read_obs_csv(path, names, start, T, dt_hours=1):
@@ -94,9 +105,11 @@ def twin_observations(cfgs, base, truth, f_dev, quantity, kw):
     from topoflow_glacier_b200.engine import MeltEngine
 
     C, T = len(cfgs), f_dev.shape[0]
+    adjust = {k: np.array([t[k] for t in truth]) for k in FORCING_DRAW if k in truth[0]}
     eng = MeltEngine({k: np.array([float(getattr(c, k)) for c in cfgs]) for k in STATIC_KEYS}, base, cfgs[0].start_time,
                      forcing_index=np.arange(C, dtype=np.int32), n_forcing_cols=C,
-                     cell_params={k: np.array([t[k] for t in truth]) for k in CELL_PARAM_KEYS}, **kw)
+                     cell_params={k: np.array([t[k] for t in truth]) for k in CELL_PARAM_KEYS},
+                     forcing_adjust=adjust or None, **kw)
     eng.set_objective(quantity, np.full((T, C), np.nan))   # selects the candidates' kernel; nothing is scored
     obs = torch.empty(T, C, dtype=torch.float64, device=f_dev.device)
     for t in range(T):
@@ -109,7 +122,7 @@ def twin_observations(cfgs, base, truth, f_dev, quantity, kw):
 
 
 def run(sets: int = 256, mode: str = "f64_fast", quantity: str = "M_total", daily: bool = False, obs_csv=None,
-        write_obs=None, seed: int = 0, verbose: bool = True) -> dict:
+        write_obs=None, seed: int = 0, verbose: bool = True, forcing_params: bool = False) -> dict:
     import torch
 
     from topoflow_glacier_b200.engine import MeltEngine
@@ -139,14 +152,16 @@ def run(sets: int = 256, mode: str = "f64_fast", quantity: str = "M_total", dail
     # the observations: one of them, at a seeded index, is the twin experiment's truth (with real observations just
     # one more uniform draw), so a run from a CSV of the twin's observations scores the same candidates.
     rng = np.random.default_rng(seed)
-    cand = [draw(rng, K) for _ in range(C)]
-    truth = [{k: float(v[0]) for k, v in draw(rng, 1).items()} for _ in range(C)]
+    cand = [draw(rng, K, forcing_params) for _ in range(C)]
+    truth = [{k: float(v[0]) for k, v in draw(rng, 1, forcing_params).items()} for _ in range(C)]
     truth_idx = rng.integers(0, K, C)
+    keys = tuple(cand[0])
     for c in range(C):
-        for k in CELL_PARAM_KEYS:
+        for k in keys:
             cand[c][k][truth_idx[c]] = truth[c][k]
     cells = {k: np.repeat([float(getattr(c, k)) for c in cfgs], K) for k in STATIC_KEYS}
     params = {k: np.concatenate([cand[c][k] for c in range(C)]) for k in CELL_PARAM_KEYS}
+    adjust = {k: np.concatenate([cand[c][k] for c in range(C)]) for k in FORCING_DRAW if k in keys}
     col = np.repeat(np.arange(C, dtype=np.int32), K)
 
     # observations [T, C]
@@ -159,7 +174,8 @@ def run(sets: int = 256, mode: str = "f64_fast", quantity: str = "M_total", dail
     if write_obs:
         write_obs_csv(write_obs, obs, names, start)
 
-    eng = MeltEngine(cells, base, cfgs[0].start_time, forcing_index=col, n_forcing_cols=C, cell_params=params, **kw)
+    eng = MeltEngine(cells, base, cfgs[0].start_time, forcing_index=col, n_forcing_cols=C, cell_params=params,
+                     forcing_adjust=adjust or None, **kw)
     eng.set_objective(quantity, obs)                      # obs_index: the forcing map (one column per catchment)
     eng.run(f_dev)
     sc = {k: v.cpu().numpy() for k, v in eng.scores().items()}
@@ -170,11 +186,12 @@ def run(sets: int = 256, mode: str = "f64_fast", quantity: str = "M_total", dail
     for c in range(C):
         nse = sc["nse"][c * K:(c + 1) * K]
         i = int(np.argmax(np.where(np.isnan(nse), -np.inf, nse)))
-        best.append({"catchment": names[c], "index": i, "params": {k: float(cand[c][k][i]) for k in CELL_PARAM_KEYS},
+        best.append({"catchment": names[c], "index": i, "params": {k: float(cand[c][k][i]) for k in keys},
                      **{s: float(sc[s][c * K + i]) for s in ("n", "nse", "kge", "rmse", "bias")}})
     if verbose:
         print(f"{C} catchments x {K} candidates, {T} steps, mode {mode}, objective {quantity}"
-              f"{' (daily observations)' if daily else ''}{', column terms' if column_terms else ''}")
+              f"{' (daily observations)' if daily else ''}{', forcing parameters' if forcing_params else ''}"
+              f"{', column terms' if column_terms else ''}")
         for c, b in enumerate(best):
             tag = "" if obs_csv is not None else f"  truth at {int(truth_idx[c])}"
             print(f"{b['catchment']}: best {b['index']:4d}  NSE {b['nse']:.6f}  KGE {b['kge']:.6f}  RMSE {b['rmse']:.3e}"
@@ -193,8 +210,9 @@ def main(argv=None):
     ap.add_argument("--obs", default=None)
     ap.add_argument("--write-obs", default=None)
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--forcing-params", action="store_true")
     a = ap.parse_args(argv)
-    run(a.sets, a.mode, a.quantity, a.daily, a.obs, a.write_obs, a.seed)
+    run(a.sets, a.mode, a.quantity, a.daily, a.obs, a.write_obs, a.seed, forcing_params=a.forcing_params)
 
 
 if __name__ == "__main__":

@@ -228,6 +228,35 @@ typedef struct tfg_objective {
  * error nothing is bound and tfg_last_error() names the field.  The arrays are read by every later tfg_run.        */
 TFG_API int tfg_bind_objective(tfg_ctx* ctx, const tfg_objective* o, void* stream);
 
+/* Optional per-cell forcing adjustments: each field is a dev float64 array of length n_cells (in every mode), or NULL
+ * for the identity (offset 0, multiplier 1).  At every step cell i reads its forcing -- its own column, or column
+ * forcing_col[i] with a forcing map -- and then uses
+ *   T_air' = T_air + T_air_offset[i]      [degC + K]
+ *   P'     = P * P_multiplier[i]          [m/h]
+ * each ONE IEEE operation in the context's element type; the library rounds the offsets and multipliers to that type
+ * once, at bind time (float64 in both float64 modes, float32 in TFG_F32).  A run with adjustments is therefore
+ * bit-identical to a run whose per-cell forcing was adjusted in advance with the same two operations.  P_air, Hum_sp
+ * and uz are NOT adjusted: air pressure and humidity stay what the forcing says (the cell's own air pressure at its
+ * elevation is formed from a_elev, as without adjustments).  The adjusted values are what every later operation sees,
+ * including the fast float64 mode's test for physically sane forcings and its strict fallback: an offset that takes
+ * |T_air'| to 90 degC or more, or a multiplier that takes P' to 10 m/h or more, takes the strict step, as the same
+ * forcing given per cell would.  A cell with offset 0 and multiplier 1 gets the bits of an unbound run, except that a
+ * forcing T_air of -0.0 becomes +0.0 (IEEE: -0.0 + 0.0 = +0.0).  Ranges: T_air_offset [-30, 30] K (a 4.5 km band at
+ * 6.5 K/km; elevation bands: T_air_offset = -T_lapse_rate * (elev_cell - elev_series)), P_multiplier [0, 10].  The
+ * input values a caller sets (the forcing block, the BMI input variables) are not changed; the adjustment happens
+ * inside the step.  With adjustments bound the TFG_OPT_COLUMN_TERMS pass is not taken (the forcing-only terms then
+ * differ per cell).                                                                                                  */
+typedef struct tfg_forcing_adjust {
+  const double* T_air_offset;  /* dev float64 [n_cells] or NULL (0) */
+  const double* P_multiplier;  /* dev float64 [n_cells] or NULL (1) */
+} tfg_forcing_adjust;
+/* Bind (a != NULL) or unbind (a == NULL) forcing adjustments; call after tfg_bind_static (binding statics again unbinds
+ * them).  May be called between launches.  The library checks every value on the device, on `stream`, and waits for
+ * that check: a non-finite value or one outside the ranges above is an error, after which nothing is bound and
+ * tfg_last_error() names the field.  It then keeps the values, in its element type, in a [2][n_cells] scratch it
+ * owns; the caller's arrays are not read again.                                                                      */
+TFG_API int tfg_bind_forcing_adjust(tfg_ctx* ctx, const tfg_forcing_adjust* a, void* stream);
+
 /* host tables for steps [0, n_steps): rows[n_steps], gmt_offset_hours[n_steps][n_tz]; copied by the library
  * (each launch carries its <= 128 rows in the kernel parameter block); replaces solar.gmt_offset_hours,
  * solar_funcs.py:1616-1637, evaluated on the host                                                 */

@@ -43,6 +43,13 @@ class CellParams(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in CELL_PARAM_FIELDS]
 
 
+FORCING_ADJUST_FIELDS = ("T_air_offset", "P_multiplier")
+
+
+class ForcingAdjust(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in FORCING_ADJUST_FIELDS]
+
+
 N_OBJ = 4  # rows of Objective.acc: S_s, S_ss, S_so, S_ee
 
 
@@ -91,6 +98,7 @@ PROTOTYPES = {
     "tfg_bind_forcing_map": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64]),
     "tfg_bind_cell_params": (C.c_int, [C.c_void_p, C.POINTER(CellParams), C.c_void_p]),
     "tfg_bind_objective": (C.c_int, [C.c_void_p, C.POINTER(Objective), C.c_void_p]),
+    "tfg_bind_forcing_adjust": (C.c_int, [C.c_void_p, C.POINTER(ForcingAdjust), C.c_void_p]),
     "tfg_bind_window_carry": (C.c_int, [C.c_void_p, C.c_void_p]),
     "tfg_bind_mass_residual": (C.c_int, [C.c_void_p, C.c_void_p]),
     "tfg_bind_time": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),

@@ -26,7 +26,7 @@ import torch
 import yaml
 
 from . import _lib
-from .config import CELL_PARAM_KEYS, KERNEL_CONSTANTS, TopoflowGlacierConfig
+from .config import CELL_PARAM_KEYS, FORCING_ADJUST_KEYS, KERNEL_CONSTANTS, TopoflowGlacierConfig
 from .engine import INPUT_ROWS, MeltEngine
 from .logger import configure_logging, logger
 from .statics import CELL_KEYS
@@ -110,7 +110,8 @@ class BmiTopoflowGlacier(_BmiBase):
         ``engine_kw`` reaches ``MeltEngine``: e.g. ``mode="f64_fast"``, ``basin_id=..., n_basin=...`` or
         ``forcing_index=..., n_forcing_cols=M`` (members that share a forcing series: the input variables then hold
         ``M`` values, one per series).  Each member keeps its own ``dust_atten, canopy_factor, cloud_factor, z0_air,
-        em_surf``; members that differ in any other physical constant are refused (``ensemble_cell_params``)."""
+        em_surf`` and its own forcing adjustments ``T_air_offset`` / ``P_multiplier``; members that differ in any other
+        physical constant are refused (``ensemble_cell_params``)."""
         cfgs = []
         for c in configs:
             if isinstance(c, (str, Path)):
@@ -126,7 +127,9 @@ class BmiTopoflowGlacier(_BmiBase):
         ``base_config`` (path, dict or validated object) supplies ``dt``, the time window and the physical constants;
         ``cells`` maps the per-catchment yaml keys (``statics.CELL_KEYS``: ``da, slope, aspect, lon, lat, elev,
         h0_snow, h0_ice, h0_swe, h0_iwe, T_rain_snow``) to float64 ``[N]`` arrays, and may also give per-cell values
-        of ``config.CELL_PARAM_KEYS`` (``dust_atten`` ... ``em_surf``; the others come from ``base_config``).  ``zones`` / ``tz_idx`` as for
+        of ``config.CELL_PARAM_KEYS`` (``dust_atten`` ... ``em_surf``; the others come from ``base_config``) and of the
+        forcing adjustments ``T_air_offset`` / ``P_multiplier`` (``MeltEngine.set_forcing_adjust``; keys not given take
+        ``base_config``'s values).  ``zones`` / ``tz_idx`` as for
         ``MeltEngine``; ``engine_kw`` reaches it too (``mode``, ``basin_id``, ``n_basin``, ``forcing_index`` ...).
         With ``shard=True`` under an initialised ``torch.distributed`` group every rank keeps only its own
         128-aligned block of the cells (``sharding.shard_bounds``) -- see ``ShardedMeltEngine``."""
@@ -136,10 +139,13 @@ class BmiTopoflowGlacier(_BmiBase):
                 c = yaml.safe_load(f)
         self.cfg = c if isinstance(c, TopoflowGlacierConfig) else TopoflowGlacierConfig.model_validate(c)
         par = {k: np.atleast_1d(np.asarray(cells[k], dtype=np.float64)) for k in CELL_PARAM_KEYS if k in cells}
+        adj = {k: np.atleast_1d(np.asarray(cells[k] if k in cells else getattr(self.cfg, k), dtype=np.float64))
+               for k in FORCING_ADJUST_KEYS}
         cells = {k: np.atleast_1d(np.asarray(cells[k], dtype=np.float64)) for k in CELL_KEYS}
+        n = cells["lat"].size
         if par:
-            n = cells["lat"].size
             engine_kw.setdefault("cell_params", {k: np.broadcast_to(v, (n,)) for k, v in par.items()})
+        engine_kw.setdefault("forcing_adjust", {k: np.broadcast_to(v, (n,)) for k, v in adj.items()})
         if zones is None:
             h = self.cfg
             zones = [h.utc_offset_hours if h.utc_offset_hours is not None else
@@ -149,6 +155,8 @@ class BmiTopoflowGlacier(_BmiBase):
     def _build(self, cfgs, **engine_kw) -> None:
         head = cfgs[0]
         engine_kw.setdefault("cell_params", ensemble_cell_params(cfgs))
+        engine_kw.setdefault("forcing_adjust", {k: np.array([getattr(c, k) for c in cfgs], dtype=np.float64)
+                                                for k in FORCING_ADJUST_KEYS})
         cells = {k: np.array([getattr(c, k) for c in cfgs], dtype=np.float64) for k in CELL_KEYS}
         zones, tz_idx = [], np.zeros(len(cfgs), dtype=np.uint8)
         for i, c in enumerate(cfgs):

@@ -7,7 +7,9 @@ backwards compatible:
 * ``start_time`` / ``end_time`` given as YAML integers are coerced to ``str`` (three of the five shipped
   configs hold unquoted integers, which the reference's ``str`` field rejects);
 * optional extension keys (ignored by the reference): ``tz_name`` / ``utc_offset_hours`` (the reference looks
-  the zone up with ``timezonefinder``; here the zone is data), ``precision``, ``device``, ``ensemble``.
+  the zone up with ``timezonefinder``; here the zone is data), ``precision``, ``device``, ``ensemble``,
+  and the per-cell forcing adjustments ``T_air_offset`` [K] / ``P_multiplier`` [-] (``FORCING_ADJUST_RANGES``).  The
+  schema's legacy ``P_factor`` stays parsed and ignored, as in the reference.
 """
 
 from __future__ import annotations
@@ -17,6 +19,7 @@ from typing import Any, Optional
 from pydantic import ConfigDict, Field, create_model, field_validator
 
 __all__ = ["TopoflowGlacierConfig", "KERNEL_CONSTANTS", "CELL_PARAM_KEYS", "CELL_PARAM_RANGES", "check_cell_params",
+           "FORCING_ADJUST_KEYS", "FORCING_ADJUST_RANGES", "FORCING_ADJUST_IDENTITY", "check_forcing_adjust",
            "default_constants"]
 
 _REQ = ...  # pydantic's "required" marker
@@ -84,6 +87,8 @@ _TABLE: dict[str, tuple[type, Any, dict, str]] = {
     "precision": (str, "f64", {}, "f64 | f64_fast | f32"),
     "device": (int, 0, {}, "CUDA device ordinal"),
     "ensemble": (Optional[list], None, {}, "Further config files advanced as extra cells of the same model"),
+    "T_air_offset": (float, 0.0, {"ge": -30.0, "le": 30.0}, "Added to the forcing's air temperature [K]"),
+    "P_multiplier": (float, 1.0, {"ge": 0.0, "le": 10.0}, "Multiplies the forcing's precipitation rate [-]"),
 }
 
 # constants handed to the kernels (tfg_constants in include/tfglacier.h)
@@ -110,6 +115,27 @@ def check_cell_params(params) -> dict:
         if not bool(((v >= lo) & (v <= hi)).all()):   # NaN and +-inf compare false
             raise ValueError(f"{k}: every value must be finite and within [{lo}, {hi}]")
     return params
+
+
+# per-cell adjustments of the forcing a cell reads (MeltEngine(forcing_adjust=...), tfg_bind_forcing_adjust)
+FORCING_ADJUST_KEYS = ("T_air_offset", "P_multiplier")
+FORCING_ADJUST_RANGES = {k: (_TABLE[k][2]["ge"], _TABLE[k][2]["le"]) for k in FORCING_ADJUST_KEYS}
+FORCING_ADJUST_IDENTITY = {k: _TABLE[k][1] for k in FORCING_ADJUST_KEYS}
+
+
+def check_forcing_adjust(adjust) -> dict:
+    """Validate per-cell forcing adjustments (NumPy arrays or torch tensors, any device) against their ranges.
+
+    Returns ``adjust`` as a plain dict; raises ``ValueError`` naming the first unknown key, or the first key holding a
+    value that is not finite or outside its range."""
+    adjust = dict(adjust)
+    for k, v in adjust.items():
+        if k not in FORCING_ADJUST_RANGES:
+            raise ValueError(f"{k!r} is not a forcing adjustment (one of {', '.join(FORCING_ADJUST_KEYS)})")
+        lo, hi = FORCING_ADJUST_RANGES[k]
+        if not bool(((v >= lo) & (v <= hi)).all()):   # NaN and +-inf compare false
+            raise ValueError(f"{k}: every value must be finite and within [{lo}, {hi}]")
+    return adjust
 
 
 def _coerce_time(cls, v):  # noqa: ANN001

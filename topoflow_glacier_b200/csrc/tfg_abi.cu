@@ -61,6 +61,10 @@ struct tfg_ctx {
   tfg_objective obj{};                   // tfg_bind_objective (caller's arrays)
   bool have_obj = false;
   int* obj_bad = nullptr;                // device flag of tfg_bind_objective's range check of obs_col (owned)
+  void* fadj = nullptr;                  // [2][n_cells] T_air offset and P multiplier, context element type (owned)
+  size_t fadj_bytes = 0;
+  int* fadj_bad = nullptr;               // device flags of tfg_bind_forcing_adjust's range check (owned)
+  bool have_fadj = false;                // tfg_bind_forcing_adjust: the scratch holds this context's adjustments
 };
 
 namespace {
@@ -209,6 +213,7 @@ tfg::RunParams<raw> make_params(const tfg_ctx* x, const void* forcing, int64_t s
   p.n_basin = n_basin;
   p.k = derive<raw>(x->c);
   p.cell_par = x->have_cell_par ? static_cast<const raw*>(x->cell_par) : nullptr;
+  p.fadj = x->have_fadj ? static_cast<const raw*>(x->fadj) : nullptr;
   // objective: the scored part of [step0, step0 + n_steps) is its intersection with the observation window; a launch
   // outside the window leaves obj_acc NULL and runs the kernels without an objective
   if (x->have_obj) {
@@ -250,6 +255,18 @@ __global__ void cell_params_kernel(const tfg_cell_params in, const tfg_constants
     if (f32) static_cast<float*>(out)[r * N + i] = (float)f[r];
     else static_cast<double*>(out)[r * N + i] = f[r];
   }
+}
+
+// ---- forcing adjustments (tfg_bind_forcing_adjust): range check, then one rounding to the element type ------------
+// bit 0 of *bad: T_air_offset outside [-30, 30] K or not finite; bit 1: P_multiplier outside [0, 10] or not finite
+__global__ void forcing_adjust_kernel(const tfg_forcing_adjust in, void* out, bool f32, int64_t N, int* bad) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= N) return;
+  const double off = in.T_air_offset ? in.T_air_offset[i] : 0.0, mul = in.P_multiplier ? in.P_multiplier[i] : 1.0;
+  const int flags = (!(off >= -30.0 && off <= 30.0) ? 1 : 0) | (!(mul >= 0.0 && mul <= 10.0) ? 2 : 0);  // NaN fails too
+  if (flags) atomicOr(bad, flags);
+  if (f32) { static_cast<float*>(out)[i] = (float)off; static_cast<float*>(out)[N + i] = (float)mul; }
+  else { static_cast<double*>(out)[i] = off; static_cast<double*>(out)[N + i] = mul; }
 }
 
 // ---- objective (tfg_bind_objective): *bad = 1 if an observation column index is outside [0, n_cols) -------------
@@ -413,6 +430,8 @@ void tfg_destroy(tfg_ctx* x) {
   if (x->cell_par) cudaFree(x->cell_par);
   if (x->cell_par_bad) cudaFree(x->cell_par_bad);
   if (x->obj_bad) cudaFree(x->obj_bad);
+  if (x->fadj) cudaFree(x->fadj);
+  if (x->fadj_bad) cudaFree(x->fadj_bad);
   delete x;
 }
 
@@ -456,6 +475,43 @@ int tfg_bind_static(tfg_ctx* x, int64_t n_cells, const tfg_statics* s) {
   x->have_static = true;
   x->have_cell_par = false;  // sized for the old cell count: bind again
   x->have_obj = false;       // likewise the objective's per-cell arrays
+  x->have_fadj = false;      // and the forcing adjustments
+  return 0;
+}
+
+int tfg_bind_forcing_adjust(tfg_ctx* x, const tfg_forcing_adjust* a, void* stream) {
+  if (!x) return fail("tfg_bind_forcing_adjust: NULL context");
+  x->have_fadj = false;
+  if (!a) return 0;
+#if defined(TFG_LEAN_W2) || TFG_WS || TFG_PIPELINE || TFG_SPLIT_STEP
+  return fail("tfg_bind_forcing_adjust: this build runs an experimental kernel variant, which has no forcing adjustments");
+#endif
+  if (!x->have_static) return fail("tfg_bind_forcing_adjust: call after tfg_bind_static");
+  TFG_CUDA(cudaSetDevice(x->device));
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const size_t need = 2 * (size_t)x->n_cells * tfg_elem_size(x);
+  if (x->fadj_bytes < need) {
+    if (x->fadj) TFG_CUDA(cudaFree(x->fadj));
+    x->fadj = nullptr;
+    x->fadj_bytes = 0;
+    TFG_CUDA(cudaMalloc(&x->fadj, need));
+    x->fadj_bytes = need;
+  }
+  if (!x->fadj_bad) TFG_CUDA(cudaMalloc(&x->fadj_bad, sizeof(int)));
+  TFG_CUDA(cudaMemsetAsync(x->fadj_bad, 0, sizeof(int), s));
+  forcing_adjust_kernel<<<(unsigned)((x->n_cells + 255) / 256), 256, 0, s>>>(*a, x->fadj, x->mode == TFG_F32, x->n_cells,
+                                                                             x->fadj_bad);
+  TFG_CUDA(cudaGetLastError());
+  int bad = 0;
+  TFG_CUDA(cudaMemcpyAsync(&bad, x->fadj_bad, sizeof(int), cudaMemcpyDeviceToHost, s));
+  TFG_CUDA(cudaStreamSynchronize(s));
+  if (bad) {
+    std::string m = "tfg_bind_forcing_adjust: values not finite or outside their range:";
+    if (bad & 1) m += " T_air_offset [-30, 30]";
+    if (bad & 2) m += " P_multiplier [0, 10]";
+    return fail(m.c_str());
+  }
+  x->have_fadj = true;
   return 0;
 }
 
@@ -610,8 +666,9 @@ int tfg_run(tfg_ctx* x, const void* forcing, int64_t step0, int32_t n_steps, voi
       // step instead of redoing it per cell.  Same device functions either way: results do not depend on this switch
       // (test_column_terms_*).  Not for launches so small that a second kernel launch costs more than it saves
       // (per-step BMI updates of a few cells); the fast mode leaves SATTERLUND configurations to its strict step.
+      // Forcing adjustments make the forcing differ per cell, so the pass is not taken while they are bound.
       const size_t need = (size_t)nt * (size_t)x->n_cols * tfg::kCtCount * sizeof(double);
-      if (x->column_terms && x->forcing_col && !x->use_tma && (strict || !x->c.satterlund) && x->n_cols * 8 <= x->n_cells &&
+      if (x->column_terms && x->forcing_col && !x->have_fadj && !x->use_tma && (strict || !x->c.satterlund) && x->n_cols * 8 <= x->n_cells &&
           (int64_t)nt * x->n_cells >= 65536 && need <= (size_t(1) << 31)) {
         if (x->col_terms_bytes < need) {   // grows to the largest launch seen; a failed allocation leaves the plain path
           if (x->col_terms) cudaFree(x->col_terms);

@@ -89,7 +89,16 @@ struct RunParams {
   int32_t obj_t_lo, obj_t_hi, obj_quantity;
   double agg_lo;               // 2^L: fraction bits of the low word of exact aggregates (with agg_up; here, behind the
                                // members above, so that the kernels without aggregates keep their parameter offsets)
+  const raw* fadj;             // optional [2][n_cells] T_air offset and P multiplier (tfg_bind_forcing_adjust); last, so
+                               // that the kernels without adjustments keep their parameter offsets
 };
+
+// One IEEE operation in the element type, never contracted into a neighbouring multiply-add: the forcing adjustment
+// must give the bits of a forcing adjusted in advance (tfg_bind_forcing_adjust)
+__device__ __forceinline__ double add_once(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ float add_once(float a, float b) { return __fadd_rn(a, b); }
+__device__ __forceinline__ double mul_once(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float mul_once(float a, float b) { return __fmul_rn(a, b); }
 
 template <class raw> __device__ __forceinline__ raw ld_stream(const raw* p) { return __ldcs(p); }
 
@@ -206,7 +215,8 @@ struct ObjSums {
   }
 };
 
-template <class P, bool REC, bool AGG, bool VOL, bool TMA = false, bool PRE = false, bool PAR = false, bool OBJ = false>
+template <class P, bool REC, bool AGG, bool VOL, bool TMA = false, bool PRE = false, bool PAR = false, bool OBJ = false,
+          bool ADJ = false>
 __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f32 ? TFG_MIN_BLOCKS_F32 : TFG_MIN_BLOCKS)) run_kernel(const __grid_constant__ RunParams<typename P::raw> p) {
   using raw = typename P::raw;
   using R = Num<P>;
@@ -225,7 +235,12 @@ __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f3
   static_assert(kSmem || !PAR, "per-cell parameters live in shared memory");
   static_assert(!(PAR && TMA), "per-cell parameters run the register-prefetch kernel");
   // PAR: the per-cell surface factors in kPCount more columns (only in these instantiations: the others keep their footprint)
-  __shared__ raw sm_cell[kSmem ? kSCount + (PAR ? kPCount : 0) : 1][kBlock];
+  // ADJ: the cell's T_air offset and P multiplier in two more columns behind them, read where the forcing is read (two
+  // more registers across the time loop would cost more, in a kernel at its register limit)
+  static_assert(kSmem || !ADJ, "forcing adjustments live in shared memory");
+  static_assert(!(ADJ && (TMA || PRE)), "forcing adjustments run the register-prefetch kernel on the forcing itself");
+  constexpr int kSAdj = kSCount + (PAR ? kPCount : 0);   // column of the T_air offset; the P multiplier follows
+  __shared__ raw sm_cell[kSmem ? kSAdj + (ADJ ? 2 : 0) : 1][kBlock];
   using Cell = typename std::conditional<kSmem, SmemCell<raw, kBlock, PAR>, RegCell<raw>>::type;
   Cell s;
   if constexpr (kSmem) s.base = (unsigned)__cvta_generic_to_shared(&sm_cell[0][threadIdx.x]);
@@ -233,6 +248,7 @@ __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f3
 #pragma unroll
     for (int i = 0; i < kPCount; ++i) s.set(kSCount + i, __ldg(p.cell_par + (int64_t)i * p.n_cells + c));
   }
+  if constexpr (ADJ) { s.set(kSAdj, __ldg(p.fadj + c)); s.set(kSAdj + 1, __ldg(p.fadj + p.n_cells + c)); }
   s.set(kSaElev, __ldg(p.a_elev + c)); s.set(kSSinLat, __ldg(p.sin_lat + c)); s.set(kSCosLat, __ldg(p.cos_lat + c));
   s.set(kSNegTanLat, __ldg(p.neg_tan_lat + c)); s.set(kSSinEq, __ldg(p.sin_eq + c)); s.set(kSCosEq, __ldg(p.cos_eq + c));
   s.set(kSNegTanEq, __ldg(p.neg_tan_eq + c)); s.set(kSDlon, __ldg(p.dlon + c)); s.set(kSTNoon, __ldg(p.t_noon + c));
@@ -404,6 +420,10 @@ __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f3
       f0 = sm_next[t & 1][0][threadIdx.x]; f1 = sm_next[t & 1][1][threadIdx.x]; f2 = sm_next[t & 1][2][threadIdx.x];
       f3 = sm_next[t & 1][3][threadIdx.x]; f4 = sm_next[t & 1][4][threadIdx.x];
       if (t + 1 < p.n_steps) stage_forcing(t + 1);
+    }
+    if constexpr (ADJ) {  // T_air' = T_air + offset, P' = P * multiplier: what the sanity test and both steps see
+      f1 = add_once(f1, s.get(kSAdj));
+      f0 = mul_once(f0, s.get(kSAdj + 1));
     }
     if constexpr (PRE && !TFG_CT_REGPF) { if (t > 0) load_line(f + (int64_t)t * (kCtCount * FN), f0, f1, f2, f3, f4, e0, e1, e2); }
     const TimeRow<raw>& row = p.rows[t];
@@ -678,6 +698,18 @@ cudaError_t launch_run_as(const RunParams<typename P::raw>& p, bool rec, bool ag
                    ((reinterpret_cast<uintptr_t>(p.forcing) & 15) == 0) &&
                    ((p.n_cells * sizeof(typename P::raw)) % 16 == 0);
   const size_t dyn = P::lean ? fm::kTabDoubles * sizeof(double) : 0;
+  if (p.fadj != nullptr) {
+    // forcing adjustments bound: the two kernel shapes of the objective, with and without it (tfg_run never binds
+    // column terms then: the forcing-only terms differ per cell)
+    if (p.obj_acc != nullptr) {
+      if (rec) run_kernel<P, true, true, true, false, false, PAR, true, true><<<grid, kBlock, dyn, stream>>>(p);
+      else run_kernel<P, false, true, true, false, false, PAR, true, true><<<grid, kBlock, dyn, stream>>>(p);
+    } else {
+      if (rec) run_kernel<P, true, true, true, false, false, PAR, false, true><<<grid, kBlock, dyn, stream>>>(p);
+      else run_kernel<P, false, true, true, false, false, PAR, false, true><<<grid, kBlock, dyn, stream>>>(p);
+    }
+    return cudaGetLastError();
+  }
   if (p.obj_acc != nullptr) {
     // objective bound: two kernel shapes only, both of which test basin_agg and vol_P at run time (register prefetch,
     // like PAR); the recording one for launches that record
@@ -719,7 +751,7 @@ cudaError_t launch_run_as(const RunParams<typename P::raw>& p, bool rec, bool ag
 }
 
 // per-cell surface parameters bound (tfg_bind_cell_params): the PAR instantiations, chosen from the input; an objective
-// bound (p.obj_acc): the OBJ instantiations (launch_run_as)
+// bound (p.obj_acc): the OBJ instantiations; forcing adjustments bound (p.fadj): the ADJ instantiations (launch_run_as)
 template <class P>
 cudaError_t launch_run(const RunParams<typename P::raw>& p, bool rec, bool agg, bool vol, cudaStream_t stream) {
   return p.cell_par != nullptr ? launch_run_as<P, true>(p, rec, agg, vol, stream) : launch_run_as<P, false>(p, rec, agg, vol, stream);

@@ -18,7 +18,8 @@ import pandas as pd
 import torch
 
 from . import _lib
-from .config import CELL_PARAM_KEYS, KERNEL_CONSTANTS, check_cell_params
+from .config import (CELL_PARAM_KEYS, FORCING_ADJUST_IDENTITY, FORCING_ADJUST_KEYS, KERNEL_CONSTANTS, check_cell_params,
+                     check_forcing_adjust)
 from .statics import cell_tables
 from .timebase import parse_start, time_tables, utc_offsets
 
@@ -56,6 +57,9 @@ class MeltEngine:
         z0_air, em_surf``) to per-cell ``[N]`` arrays or device tensors: every cell runs with its own values (a
         parameter ensemble, e.g. one calibration candidate per cell); keys it does not name take the value of
         ``consts``.  See ``set_cell_params``.
+    forcing_adjust : optional mapping of ``T_air_offset`` [K] and/or ``P_multiplier`` [-] to per-cell ``[N]`` arrays or
+        device tensors: every cell adds its offset to the air temperature and multiplies the precipitation rate it
+        reads (its own forcing column or, with ``forcing_index``, its catchment's).  See ``set_forcing_adjust``.
     mode : ``"f64"`` (strict), ``"f64_fast"`` or ``"f32"``
     horizon_steps : number of steps the host time tables are prepared for (extended on demand)
     """
@@ -65,7 +69,8 @@ class MeltEngine:
                  basin_id: Optional[np.ndarray] = None, n_basin: int = 0, mode: str = "f64", device: int = 0,
                  horizon_steps: int = 24 * 366, diag_integrals: bool = True, device_statics: Optional[dict] = None,
                  tma_staging: Optional[bool] = None, forcing_index=None, n_forcing_cols: Optional[int] = None,
-                 column_terms: Optional[bool] = None, cell_params: Optional[Mapping] = None):
+                 column_terms: Optional[bool] = None, cell_params: Optional[Mapping] = None,
+                 forcing_adjust: Optional[Mapping] = None):
         self.lib = _lib.load()
         self.device = _require_cuda(device)
         self.mode = _lib.MODE_NAMES[mode] if isinstance(mode, str) else int(mode)
@@ -124,6 +129,9 @@ class MeltEngine:
             self.cell_params = None
             if cell_params is not None:
                 self.set_cell_params(cell_params)
+            self.forcing_adjust = None
+            if forcing_adjust is not None:
+                self.set_forcing_adjust(forcing_adjust)
             self.n_cols, self.forcing_index = N, None
             if forcing_index is not None:
                 self.set_forcing_map(forcing_index, n_forcing_cols, _alloc_inputs=False)
@@ -182,6 +190,37 @@ class MeltEngine:
             # the library derives its own copy on the current stream and waits for its range check
             _lib.check(self.lib.tfg_bind_cell_params(self.ctx, C.byref(p), self.stream_ptr), "tfg_bind_cell_params")
         self.cell_params = bound
+
+    def set_forcing_adjust(self, adjust: Optional[Mapping]) -> None:
+        """Bind per-cell forcing adjustments (``None`` unbinds them); may be called between launches.
+
+        ``adjust`` maps ``T_air_offset`` (K, in [-30, 30]) and/or ``P_multiplier`` (in [0, 10]) to ``[N]`` arrays or
+        tensors.  At every step cell ``i`` then uses ``T_air + T_air_offset[i]`` and ``P * P_multiplier[i]`` of the
+        forcing it reads, one operation each in the engine's float type -- the bits of a per-cell forcing adjusted in
+        advance.  ``P_air``, ``Hum_sp`` and ``uz`` are not adjusted, and the input block keeps what the caller set.
+        Values are range-checked (``ValueError``).  A key whose values are all the identity (0, 1) is not bound, and
+        with no key left the engine runs exactly as without adjustments.  Elevation bands that share a catchment's
+        series: ``T_air_offset = -T_lapse_rate * (elev_cell - elev_series)``.  Adjustments are bindings, like
+        ``set_cell_params``: ``state_dict`` does not hold them."""
+        tensors = {k: (v if torch.is_tensor(v) else torch.as_tensor(np.array(v, dtype=np.float64)))
+                   .to(self.device, torch.float64).contiguous().reshape(-1) for k, v in (adjust or {}).items()}
+        bound = {}
+        for k, t in check_forcing_adjust(tensors).items():
+            if t.numel() != self.N:
+                raise ValueError(f"{k}: one value per cell ({self.N}) expected, got {t.numel()}")
+            if not bool((t == FORCING_ADJUST_IDENTITY[k]).all()):
+                bound[k] = t
+        with torch.cuda.device(self.device):
+            if not bound:
+                _lib.check(self.lib.tfg_bind_forcing_adjust(self.ctx, None, self.stream_ptr), "tfg_bind_forcing_adjust")
+                self.forcing_adjust = None
+                return
+            a = _lib.ForcingAdjust()
+            for k in FORCING_ADJUST_KEYS:
+                setattr(a, k, bound[k].data_ptr() if k in bound else None)
+            # the library copies the values on the current stream and waits for its range check
+            _lib.check(self.lib.tfg_bind_forcing_adjust(self.ctx, C.byref(a), self.stream_ptr), "tfg_bind_forcing_adjust")
+        self.forcing_adjust = bound
 
     # ---- objective: scores of every cell against observations, accumulated inside the melt kernel ----------------
     def set_objective(self, quantity: Optional[str], obs=None, obs_step0: int = 0, obs_index=None) -> None:

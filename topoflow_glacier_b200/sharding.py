@@ -211,12 +211,12 @@ class ShardedMeltEngine:
     tables keyed like ``tfg_statics`` + ``h0_*``) for grids too large to materialise on every rank; then pass
     ``n_total``.  ``basin_id`` / ``tz_idx`` / ``forcing_index`` are global arrays (or callables ``(lo, hi)``); so is
     ``cell_params``: a mapping of global per-cell parameter arrays (``MeltEngine(cell_params=...)``), sliced here, or a
-    callable ``(lo, hi) -> mapping`` of the shard's arrays.
+    callable ``(lo, hi) -> mapping`` of the shard's arrays; ``forcing_adjust`` likewise (``MeltEngine(forcing_adjust=...)``).
     Attribute access falls through to the local ``MeltEngine`` (``state``, ``row``, ``step_index`` ...).
     """
 
     def __init__(self, cells, consts, start_time, *, n_total: Optional[int] = None, basin_id=None, n_basin: int = 0,
-                 tz_idx=None, forcing_index=None, cell_params=None, group=None, exact: bool = True,
+                 tz_idx=None, forcing_index=None, cell_params=None, forcing_adjust=None, group=None, exact: bool = True,
                  device: Optional[int] = None, **kw):
         import os
 
@@ -246,11 +246,15 @@ class ShardedMeltEngine:
             device = int(os.environ.get("LOCAL_RANK", self.rank)) % max(torch.cuda.device_count(), 1)
         if cell_params is not None:
             cell_params = cell_params(lo, hi) if callable(cell_params) else {k: v[lo:hi] for k, v in cell_params.items()}
+        if forcing_adjust is not None:
+            forcing_adjust = (forcing_adjust(lo, hi) if callable(forcing_adjust)
+                              else {k: v[lo:hi] for k, v in forcing_adjust.items()})
         dev_tables = "a_elev" in local
         self.exact = bool(exact)
         self.engine = MeltEngine(None if dev_tables else local, consts, start_time, basin_id=part(basin_id),
                                  n_basin=n_basin, tz_idx=part(tz_idx), forcing_index=part(forcing_index), device=device,
-                                 device_statics=local if dev_tables else None, cell_params=cell_params, **kw)
+                                 device_statics=local if dev_tables else None, cell_params=cell_params,
+                                 forcing_adjust=forcing_adjust, **kw)
         self._aggs: dict = {}
 
     def __getattr__(self, name):
