@@ -89,11 +89,17 @@ template <class P> __device__ __forceinline__ Num<P> fnmadd(Num<P> a, Num<P> b, 
   else return Num<P>(fma(-a.v, b.v, c.v));
 }
 
-// np.minimum / np.maximum propagate NaN; fmin/fmax do not.  Strict mode keeps NumPy's behaviour.
+// np.minimum / np.maximum propagate NaN; fmin/fmax do not.  Strict mode keeps NumPy's behaviour.  float32: PTX
+// max/min.NaN (FMNMX.NAN), one instruction that returns NaN if either operand is NaN and fmaxf/fminf's result otherwise
+// -- the float32 kernel has no strict fallback, so a missing forcing must poison the cell through these as in the
+// reference.  The fast float64 mode needs no NaN rule here: its non-finite inputs take the strict step.
 template <class P> __device__ __forceinline__ Num<P> nmax(Num<P> a, Num<P> b) {
   if constexpr (P::strict) return Num<P>((a.v >= b.v) ? a.v : ((b.v > a.v) ? b.v : a.v + b.v));
-  else if constexpr (P::f32) return Num<P>(fmaxf(a.v, b.v));
-  else {
+  else if constexpr (P::f32) {
+    float r;
+    asm("max.ftz.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a.v), "f"(b.v));
+    return Num<P>(r);
+  } else {
     // setp + selp (3 instructions).  Written in PTX because nvcc turns `a > b ? a : b` back into fmax(), whose
     // NaN canonicalisation costs 6 instructions, two of them on the FP64 pipe.
     double r;
@@ -103,8 +109,11 @@ template <class P> __device__ __forceinline__ Num<P> nmax(Num<P> a, Num<P> b) {
 }
 template <class P> __device__ __forceinline__ Num<P> nmin(Num<P> a, Num<P> b) {
   if constexpr (P::strict) return Num<P>((a.v <= b.v) ? a.v : ((b.v < a.v) ? b.v : a.v + b.v));
-  else if constexpr (P::f32) return Num<P>(fminf(a.v, b.v));
-  else {
+  else if constexpr (P::f32) {
+    float r;
+    asm("min.ftz.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a.v), "f"(b.v));
+    return Num<P>(r);
+  } else {
     double r;
     asm("{ .reg .pred p; setp.lt.f64 p, %1, %2; selp.f64 %0, %1, %2, p; }" : "=d"(r) : "d"(a.v), "d"(b.v));
     return Num<P>(r);

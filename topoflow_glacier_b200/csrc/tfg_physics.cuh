@@ -97,20 +97,22 @@ struct CellState {
 
 // float32 mode: one water-equivalent balance in float64.  h (+ low part) gains `gain`, then loses min(M*3600, h)/3600*dt*3600;
 // returns the melt rate actually realised.  Same operation order as the reference, so the melt-out residue logic carries over.
+// A NaN in h, gain or M (missing forcing: there is no strict fallback in this mode) gives a NaN depth and melt rate, as
+// the reference's np.minimum / np.maximum do.
 __device__ __forceinline__ float balance64(float& h, float& lo, float gain, float M, float dt) {
-  if (gain == 0.0f && M == 0.0f) return 0.0f;   // nothing enters or leaves (frozen pack, snow-covered ice): h + lo stays as it is
+  if (gain == 0.0f && M == 0.0f) return (h != h) ? h : 0.0f;   // nothing enters or leaves (frozen pack, snow-covered ice): h + lo stays as it is
   // single-rounding intrinsics throughout: this translation unit allows FMA contraction, and a fused w - (m dt) 3600
   // would return the rounding residue of the product instead of the reference's exact zero at melt-out
   double w = __dadd_rn((double)h, (double)lo);
   w = __dadd_rn(w, (double)gain);
   const double s3 = __dmul_rn((double)M, 3600.0);
-  const double s = (s3 < w) ? s3 : w;                 // both finite and >= 0 here: no NaN handling needed
+  const double s = (s3 < w) ? s3 : ((s3 != s3) ? s3 : w);   // min(M*3600, h), NaN if either is NaN
   // s / 3600 correctly rounded (Markstein, as div3600 in tfg_num.cuh): the reference's own float64 operations in its
   // own order, so a pack that melts out leaves a rounding residue exactly when the reference's would
   const double y = 1.0 / 3600.0, q = __dmul_rn(s, y);
   const double m = __fma_rn(__fma_rn(-3600.0, q, s), y, q);
   w = __dsub_rn(w, __dmul_rn(__dmul_rn(m, (double)dt), 3600.0));
-  w = (w > 0.0) ? w : 0.0;
+  w = (w > 0.0 || w != w) ? w : 0.0;                  // max(w, 0), NaN stays NaN
   h = (float)w;
   lo = (float)__dsub_rn(w, (double)h);
   return (float)m;
@@ -657,7 +659,7 @@ __device__ __forceinline__ void cell_step(const Consts<typename P::raw>& k, cons
   const bool is_rain = T_air > R(s.get(kSTrs));
   const bool is_snow = T_air <= R(s.get(kSTrs));
   R P_rain, P_snow;
-  if constexpr (P::strict) {
+  if constexpr (P::strict || P::f32) {   // float32 has no strict fallback: 0 for a NaN T_air, NaN for a NaN P
     P_rain = Pp * R(is_rain ? 1.0 : 0.0);
     P_snow = Pp * R(is_snow ? 1.0 : 0.0);
   } else {
@@ -878,7 +880,7 @@ __device__ __forceinline__ void cell_step(const Consts<typename P::raw>& k, cons
     tot = R(window_sum(ring_new.v));                           // :1027-1037
     n = R(st.n_days);
     const R thr = LIT(snow_thr, 0.03);
-    if constexpr (P::strict) {
+    if constexpr (P::strict || P::f32) {                      // a NaN total (missing precipitation) leaves n as it is
       n = sel(tot >= thr, R(0.0), n);                         // :1040
       n = sel(tot < thr, n + R(k.days_per_dt), n);            // :1041
     } else {
