@@ -257,6 +257,52 @@ typedef struct tfg_forcing_adjust {
  * owns; the caller's arrays are not read again.                                                                      */
 TFG_API int tfg_bind_forcing_adjust(tfg_ctx* ctx, const tfg_forcing_adjust* a, void* stream);
 
+/* Optional stochastic forcing perturbations (ensemble members): an additive, temporally correlated air-temperature error
+ * and a multiplicative, mean-preserving, log-normal precipitation error per STREAM.  Cells that share a stream get the
+ * same noise (an ensemble member spread over several cells is perturbed coherently); streams are independent.  For the
+ * stream with global id g and absolute step s >= s0 (= step0):
+ *   (w0,w1,w2,w3) = Philox4x32-10(counter = (lo32 g, hi32 g, s, 0x4E4F4953), key = (lo32 seed, hi32 seed))
+ *   u_a = (((w0 << 21) | (w1 >> 11)) + 1) * 2^-53          in (0, 1]   (53-bit integers, w widened to 64 bits)
+ *   u_b =  ((w2 << 21) | (w3 >> 11))      * 2^-53          in [0, 1)
+ *   r = sqrt(-2 ln u_a);  e_T = r cospi(2 u_b);  e_P = r sinpi(2 u_b)
+ *   z(s0) = e(s0);  z(s) = rho z(s-1) + c e(s),  c = sqrt(1 - rho^2)   (per quantity, c formed once on the host)
+ *   dT(s) = sd_T z_T(s);   fP(s) = exp(sd_P z_P(s) - sd_P^2 / 2)         (E[fP] = 1 at every step)
+ * The fourth counter word keeps these draws apart from tfg_synth_forcing's (cell, step, 0..2) counters.  Everything is
+ * float64 with libdevice log / sqrt / sincospi / exp in EVERY mode, each + - x one rounding, so the series does not
+ * depend on the translation unit or on contraction; dT and fP are rounded to the context's element type once.  Cell i
+ * at step s then uses
+ *   T_air' = (T_air + T_air_offset[i]) + dT(s)      P' = (P * P_multiplier[i]) * fP(s)
+ * of its stream, each one IEEE operation in the element type, after the forcing adjustment (tfg_bind_forcing_adjust;
+ * the identity when none is bound).  As with the adjustments, the perturbed values are what the fast mode's sanity test
+ * and its strict fallback see; the input block and the BMI input variables keep what the caller set; P_air, Hum_sp and
+ * uz are not perturbed, and the TFG_OPT_COLUMN_TERMS pass is not taken while noise is bound.
+ * Ranges: T_air_sd [0, 5] K, P_sd [0, 1.5], T_air_rho and P_rho [0, 1] (rho = 1: a constant random bias per stream),
+ * stream ids >= 0, cell_stream in [0, n_streams), step0 >= 0, steps s < 2^32.  A launch that starts before step0 is
+ * refused.
+ * The noise is a pure function of (seed, g, s0, s).  The library caches each stream's last z and the step it belongs
+ * to; a launch that does not continue from that step (a rewound checkpoint, another caller's step range) first
+ * regenerates z from s0.  Results therefore do not depend on the launch split, the per-step path, sharding, or
+ * checkpoint and rewind.                                                                                              */
+typedef struct tfg_forcing_noise {
+  uint64_t seed;
+  int64_t step0;                 /* s0: absolute step of z(s0) = e(s0)                                               */
+  double T_air_sd, T_air_rho;    /* sd_T [K], rho_T                                                                  */
+  double P_sd, P_rho;            /* sd_P (sd of ln fP), rho_P                                                        */
+  int64_t n_streams;
+  const int64_t* stream_id;      /* dev [n_streams] global ids (the Philox counter), or NULL (0 .. n_streams-1)     */
+  const int32_t* cell_stream;    /* dev [n_cells] indices into stream_id, or NULL (cell i reads stream i)            */
+} tfg_forcing_noise;
+/* Bind (n != NULL) or unbind (n == NULL) forcing noise; call after tfg_bind_static (binding statics again unbinds it).
+ * May be called between launches.  The host fields are checked on the host, stream ids and cell_stream on the device,
+ * on `stream`, and the call waits for that check: on error nothing is bound and tfg_last_error() names the field.  The
+ * library copies both arrays.  Each launch runs a pre-pass, one thread per stream, that writes the launch's dT and fP
+ * into a [n_steps][2][n_streams] scratch the library owns; where n_streams x steps would exceed 2 GB of scratch,
+ * tfg_run splits the launch into shorter ones (bit-identical: the split does not matter).                           */
+TFG_API int tfg_bind_forcing_noise(tfg_ctx* ctx, const tfg_forcing_noise* n, void* stream);
+/* The bound noise's series for absolute steps [step0, step0 + n_steps): dev dT and fP, [n_steps][n_streams] each, in
+ * the context's element type, regenerated from s0 -- the values tfg_run applies.  Does not touch the launches' cache. */
+TFG_API int tfg_forcing_noise_series(tfg_ctx* ctx, int64_t step0, int32_t n_steps, void* dT, void* fP, void* stream);
+
 /* host tables for steps [0, n_steps): rows[n_steps], gmt_offset_hours[n_steps][n_tz]; copied by the library
  * (each launch carries its <= 128 rows in the kernel parameter block); replaces solar.gmt_offset_hours,
  * solar_funcs.py:1616-1637, evaluated on the host                                                 */
@@ -274,6 +320,7 @@ TFG_API int tfg_bind_time(tfg_ctx* ctx, const tfg_time_row* rows, const double* 
  *                replaces np.sum(...) at :567-568,:1486-1494 and the driver-side `* da_m2`
  *                (examples/run_topoflow_glacier.py:115); int64 fixed-point accumulators under TFG_OPT_EXACT_AGG
  * With an objective bound (tfg_bind_objective), the steps of [step0, step0 + n_steps) inside its window are scored.
+ * With forcing noise bound (tfg_bind_forcing_noise), step0 must not be before the noise's step0.
  * n_steps == 1 re-sums the snowfall window exactly every step (the literal update()).          */
 TFG_API int tfg_run(tfg_ctx* ctx, const void* forcing, int64_t step0, int32_t n_steps, void* record, uint64_t record_mask,
             void* basin_agg, int32_t n_basin, void* stream);

@@ -50,6 +50,12 @@ class ForcingAdjust(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in FORCING_ADJUST_FIELDS]
 
 
+class ForcingNoise(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("step0", C.c_int64), ("T_air_sd", C.c_double), ("T_air_rho", C.c_double),
+                ("P_sd", C.c_double), ("P_rho", C.c_double), ("n_streams", C.c_int64), ("stream_id", C.c_void_p),
+                ("cell_stream", C.c_void_p)]
+
+
 N_OBJ = 4  # rows of Objective.acc: S_s, S_ss, S_so, S_ee
 
 
@@ -99,6 +105,8 @@ PROTOTYPES = {
     "tfg_bind_cell_params": (C.c_int, [C.c_void_p, C.POINTER(CellParams), C.c_void_p]),
     "tfg_bind_objective": (C.c_int, [C.c_void_p, C.POINTER(Objective), C.c_void_p]),
     "tfg_bind_forcing_adjust": (C.c_int, [C.c_void_p, C.POINTER(ForcingAdjust), C.c_void_p]),
+    "tfg_bind_forcing_noise": (C.c_int, [C.c_void_p, C.POINTER(ForcingNoise), C.c_void_p]),
+    "tfg_forcing_noise_series": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "tfg_bind_window_carry": (C.c_int, [C.c_void_p, C.c_void_p]),
     "tfg_bind_mass_residual": (C.c_int, [C.c_void_p, C.c_void_p]),
     "tfg_bind_time": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),

@@ -20,7 +20,7 @@ from pydantic import ConfigDict, Field, create_model, field_validator
 
 __all__ = ["TopoflowGlacierConfig", "KERNEL_CONSTANTS", "CELL_PARAM_KEYS", "CELL_PARAM_RANGES", "check_cell_params",
            "FORCING_ADJUST_KEYS", "FORCING_ADJUST_RANGES", "FORCING_ADJUST_IDENTITY", "check_forcing_adjust",
-           "default_constants"]
+           "FORCING_NOISE_RANGES", "check_forcing_noise", "default_constants"]
 
 _REQ = ...  # pydantic's "required" marker
 
@@ -136,6 +136,49 @@ def check_forcing_adjust(adjust) -> dict:
         if not bool(((v >= lo) & (v <= hi)).all()):   # NaN and +-inf compare false
             raise ValueError(f"{k}: every value must be finite and within [{lo}, {hi}]")
     return adjust
+
+
+# stochastic forcing perturbations of ensemble members (MeltEngine(forcing_noise=...), tfg_bind_forcing_noise)
+FORCING_NOISE_RANGES = {"T_air_sd": (0.0, 5.0), "T_air_rho": (0.0, 1.0), "P_sd": (0.0, 1.5), "P_rho": (0.0, 1.0)}
+_NOISE_STEP_LIMIT = 2**32   # a step is one 32-bit word of the Philox counter
+
+
+def check_forcing_noise(noise) -> dict:
+    """Validate a forcing-noise mapping: ``seed`` (required, an integer in [0, 2^64)), the scalars of
+    ``FORCING_NOISE_RANGES`` (``T_air_sd`` [K], ``T_air_rho``, ``P_sd``, ``P_rho``; absent ones are 0), an optional
+    per-cell ``stream`` of global stream ids >= 0 (NumPy array or torch tensor, any device) and an optional ``step0``
+    in [0, 2^32).
+
+    Returns a new dict with the scalars as floats, ``seed`` and ``step0`` as ints and ``stream`` as given; raises
+    ``ValueError`` naming the first unknown key or the first field that is missing, not finite or outside its range."""
+    noise = dict(noise)
+    allowed = set(FORCING_NOISE_RANGES) | {"seed", "stream", "step0"}
+    for k in noise:
+        if k not in allowed:
+            raise ValueError(f"{k!r} is not a forcing-noise key (one of {', '.join(sorted(allowed))})")
+    out = {}
+    for k, (lo, hi) in FORCING_NOISE_RANGES.items():
+        v = float(noise.get(k, 0.0))
+        if not lo <= v <= hi:   # NaN and +-inf compare false
+            raise ValueError(f"{k}: must be finite and within [{lo}, {hi}], got {v!r}")
+        out[k] = v
+    if "seed" not in noise:
+        raise ValueError("seed: required (an integer in [0, 2^64))")
+    seed = noise["seed"]
+    if isinstance(seed, bool) or int(seed) != seed or not 0 <= int(seed) < 2**64:
+        raise ValueError(f"seed: must be an integer in [0, 2^64), got {seed!r}")
+    out["seed"] = int(seed)
+    if noise.get("step0") is not None:
+        s0 = noise["step0"]
+        if isinstance(s0, bool) or int(s0) != s0 or not 0 <= int(s0) < _NOISE_STEP_LIMIT:
+            raise ValueError(f"step0: must be an integer in [0, 2^32), got {s0!r}")
+        out["step0"] = int(s0)
+    if noise.get("stream") is not None:
+        st = noise["stream"]
+        if not bool((st >= 0).all()):
+            raise ValueError("stream: global stream ids must be >= 0")
+        out["stream"] = st
+    return out
 
 
 def _coerce_time(cls, v):  # noqa: ANN001

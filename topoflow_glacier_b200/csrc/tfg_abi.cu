@@ -6,6 +6,8 @@
 #include <string.h>
 
 #include <algorithm>
+#include <climits>
+#include <cmath>
 #include <string>
 #include <vector>
 
@@ -65,6 +67,18 @@ struct tfg_ctx {
   size_t fadj_bytes = 0;
   int* fadj_bad = nullptr;               // device flags of tfg_bind_forcing_adjust's range check (owned)
   bool have_fadj = false;                // tfg_bind_forcing_adjust: the scratch holds this context's adjustments
+  // forcing noise (tfg_bind_forcing_noise)
+  tfg_forcing_noise noise{};             // host fields; the arrays are the library's copies below
+  bool have_noise = false;
+  double noise_c[2] = {0.0, 0.0};        // sqrt(1 - rho^2) of T_air and P, formed once here
+  int64_t* noise_ids = nullptr;          // [n_streams] global stream ids (owned)
+  int32_t* noise_cell = nullptr;         // [n_cells] stream index of each cell (owned)
+  double* noise_z = nullptr;             // [2][n_streams] z_T, z_P of step noise_next - 1 (owned)
+  int64_t noise_streams_cap = 0, noise_cells_cap = 0;
+  int64_t noise_next = -1;               // step whose z the cache continues to; -1: regenerate from step0
+  void* noise_buf = nullptr;             // [<= kMaxLaunchSteps][2][n_streams] dT, fP of a launch, element type (owned)
+  size_t noise_buf_bytes = 0;
+  int* noise_bad = nullptr;              // device flags of tfg_bind_forcing_noise's checks (owned)
 };
 
 namespace {
@@ -399,6 +413,122 @@ __global__ void synth_kernel(raw* __restrict__ out, const raw* __restrict__ elev
   }
 }
 
+// ---- forcing noise (tfg_bind_forcing_noise) -------------------------------------------------------------------------
+constexpr int64_t kNoiseStepLimit = int64_t(1) << 32;   // a step is one 32-bit counter word
+constexpr size_t kNoiseScratchCap = size_t(1) << 31;    // 2 GB of [steps][2][n_streams], as the column-term scratch
+
+struct NoiseGen {
+  uint64_t seed;
+  int64_t s0;
+  double sd_T, rho_T, c_T, sd_P, rho_P, c_P, half_var_P;   // c = sqrt(1 - rho^2), half_var_P = sd_P^2 / 2 (host)
+};
+
+// The two standard normals of stream id g at absolute step s (include/tfglacier.h states the definition)
+__device__ __forceinline__ void noise_normals(uint64_t seed, int64_t g, int64_t s, double& eT, double& eP) {
+  uint32_t w[4];
+  philox4x32_10((uint32_t)g, (uint32_t)((uint64_t)g >> 32), (uint32_t)s, 0x4E4F4953u, (uint32_t)seed,
+                (uint32_t)(seed >> 32), w);
+  const uint64_t a = ((uint64_t)w[0] << 21) | (w[1] >> 11), b = ((uint64_t)w[2] << 21) | (w[3] >> 11);
+  const double ua = (double)(a + 1) * 0x1p-53, ub = (double)b * 0x1p-53;   // exact: 53-bit integers
+  const double r = sqrt(__dmul_rn(-2.0, log(ua)));
+  double sp, cp;
+  sincospi(__dmul_rn(2.0, ub), &sp, &cp);
+  eT = __dmul_rn(r, cp);
+  eP = __dmul_rn(r, sp);
+}
+
+// One thread per stream walks absolute steps [from, step0 + n_steps) and writes dT, fP of steps >= step0 to
+// outT / outP[(s - step0) * row + j].  from == g.s0 starts the recursion at z(s0) = e(s0); from > g.s0 continues from
+// z[j], z[n_streams + j] (= z(from - 1)).  z != nullptr: the last z is stored back there.
+template <class raw>
+__global__ void __launch_bounds__(128) forcing_noise_kernel(const NoiseGen g, const int64_t* __restrict__ ids,
+                                                            int64_t n_streams, int64_t from, int64_t step0, int32_t n_steps,
+                                                            double* __restrict__ z, raw* __restrict__ outT,
+                                                            raw* __restrict__ outP, int64_t row) {
+  const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n_streams) return;
+  const int64_t id = ids[j];
+  double zT = 0.0, zP = 0.0;
+  if (from > g.s0) { zT = z[j]; zP = z[n_streams + j]; }
+  for (int64_t s = from; s < step0 + n_steps; ++s) {
+    double eT, eP;
+    noise_normals(g.seed, id, s, eT, eP);
+    if (s == g.s0) { zT = eT; zP = eP; }
+    else {
+      zT = __dadd_rn(__dmul_rn(g.rho_T, zT), __dmul_rn(g.c_T, eT));
+      zP = __dadd_rn(__dmul_rn(g.rho_P, zP), __dmul_rn(g.c_P, eP));
+    }
+    if (s >= step0) {
+      const int64_t o = (s - step0) * row + j;
+      outT[o] = (raw)__dmul_rn(g.sd_T, zT);
+      outP[o] = (raw)exp(__dadd_rn(__dmul_rn(g.sd_P, zP), -g.half_var_P));
+    }
+  }
+  if (z) { z[j] = zT; z[n_streams + j] = zP; }
+}
+
+// The library's copies of the stream ids (NULL: 0 .. n_streams-1) and of the cell -> stream map (NULL: cell i reads
+// stream i).  Bit 0 of *bad: a stream id < 0; bit 1: a cell_stream entry outside [0, n_streams)
+__global__ void noise_index_kernel(const int64_t* ids, int64_t n_streams, const int32_t* cell_stream, int64_t N,
+                                   int64_t* ids_out, int32_t* cell_out, int* bad) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < (n_streams > N ? n_streams : N);
+       i += (int64_t)gridDim.x * blockDim.x) {
+    int flags = 0;
+    if (i < n_streams) {
+      const int64_t g = ids ? ids[i] : i;
+      if (g < 0) flags |= 1;
+      ids_out[i] = g;
+    }
+    if (i < N) {
+      const int32_t k = cell_stream ? cell_stream[i] : (int32_t)i;
+      if (!(k >= 0 && (int64_t)k < n_streams)) flags |= 2;
+      cell_out[i] = k;
+    }
+    if (flags) atomicOr(bad, flags);
+  }
+}
+
+NoiseGen noise_gen(const tfg_ctx* x) {
+  const tfg_forcing_noise& n = x->noise;
+  return NoiseGen{n.seed, n.step0, n.T_air_sd, n.T_air_rho, x->noise_c[0], n.P_sd, n.P_rho, x->noise_c[1],
+                  0.5 * (n.P_sd * n.P_sd)};
+}
+
+// Steps per launch while noise is bound: the [steps][2][n_streams] scratch stays within kNoiseScratchCap
+int32_t noise_launch_steps(const tfg_ctx* x) {
+  const int64_t cap = (int64_t)(kNoiseScratchCap / ((size_t)x->noise.n_streams * 2 * tfg_elem_size(x)));
+  return (int32_t)std::max<int64_t>(1, std::min<int64_t>(tfg::kMaxLaunchSteps, cap));
+}
+
+// Noise pre-pass of one launch, on the launch's stream: dT and fP of its steps into the scratch, continuing the cached
+// z when the launch follows the last one, else regenerating it from step0.  `want_steps` sizes a new scratch.
+template <class raw>
+cudaError_t noise_pass(tfg_ctx* x, tfg::RunParams<raw>& p, int32_t want_steps, cudaStream_t s) {
+  const int64_t S = x->noise.n_streams;
+  const size_t need = (size_t)p.n_steps * 2 * (size_t)S * sizeof(raw);
+  if (x->noise_buf_bytes < need) {
+    if (x->noise_buf) cudaFree(x->noise_buf);
+    x->noise_buf = nullptr;
+    x->noise_buf_bytes = 0;
+    const size_t want = std::max<size_t>(need, (size_t)want_steps * 2 * (size_t)S * sizeof(raw));
+    cudaError_t e = cudaMalloc(&x->noise_buf, want);
+    if (e != cudaSuccess) return e;
+    x->noise_buf_bytes = want;
+  }
+  raw* buf = static_cast<raw*>(x->noise_buf);
+  const int64_t from = (x->noise_next == p.step0) ? p.step0 : x->noise.step0;
+  x->noise_next = -1;
+  forcing_noise_kernel<raw><<<(unsigned)((S + 127) / 128), 128, 0, s>>>(noise_gen(x), x->noise_ids, S, from, p.step0,
+                                                                         p.n_steps, x->noise_z, buf, buf + S, 2 * S);
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  x->noise_next = p.step0 + p.n_steps;
+  p.noise = buf;
+  p.cell_stream = x->noise_cell;
+  p.n_streams = S;
+  return cudaSuccess;
+}
+
 }  // namespace
 
 extern "C" {
@@ -432,6 +562,11 @@ void tfg_destroy(tfg_ctx* x) {
   if (x->obj_bad) cudaFree(x->obj_bad);
   if (x->fadj) cudaFree(x->fadj);
   if (x->fadj_bad) cudaFree(x->fadj_bad);
+  if (x->noise_ids) cudaFree(x->noise_ids);
+  if (x->noise_cell) cudaFree(x->noise_cell);
+  if (x->noise_z) cudaFree(x->noise_z);
+  if (x->noise_buf) cudaFree(x->noise_buf);
+  if (x->noise_bad) cudaFree(x->noise_bad);
   delete x;
 }
 
@@ -476,6 +611,87 @@ int tfg_bind_static(tfg_ctx* x, int64_t n_cells, const tfg_statics* s) {
   x->have_cell_par = false;  // sized for the old cell count: bind again
   x->have_obj = false;       // likewise the objective's per-cell arrays
   x->have_fadj = false;      // and the forcing adjustments
+  x->have_noise = false;     // and the forcing noise
+  return 0;
+}
+
+int tfg_bind_forcing_noise(tfg_ctx* x, const tfg_forcing_noise* n, void* stream) {
+  if (!x) return fail("tfg_bind_forcing_noise: NULL context");
+  x->have_noise = false;
+  if (!n) return 0;
+#if defined(TFG_LEAN_W2) || TFG_WS || TFG_PIPELINE || TFG_SPLIT_STEP
+  return fail("tfg_bind_forcing_noise: this build runs an experimental kernel variant, which has no forcing noise");
+#endif
+  if (!x->have_static) return fail("tfg_bind_forcing_noise: call after tfg_bind_static");
+  auto within = [](double v, double lo, double hi) { return v >= lo && v <= hi; };   // NaN and +-inf fail too
+  if (!within(n->T_air_sd, 0.0, 5.0)) return fail("tfg_bind_forcing_noise: T_air_sd must be finite and within [0, 5] K");
+  if (!within(n->T_air_rho, 0.0, 1.0)) return fail("tfg_bind_forcing_noise: T_air_rho must be finite and within [0, 1]");
+  if (!within(n->P_sd, 0.0, 1.5)) return fail("tfg_bind_forcing_noise: P_sd must be finite and within [0, 1.5]");
+  if (!within(n->P_rho, 0.0, 1.0)) return fail("tfg_bind_forcing_noise: P_rho must be finite and within [0, 1]");
+  if (n->step0 < 0 || n->step0 >= kNoiseStepLimit) return fail("tfg_bind_forcing_noise: step0 must be in [0, 2^32)");
+  if (n->n_streams <= 0 || n->n_streams > INT32_MAX)
+    return fail("tfg_bind_forcing_noise: n_streams must be in [1, 2^31 - 1]");
+  if (!n->cell_stream && n->n_streams != x->n_cells)
+    return fail("tfg_bind_forcing_noise: n_streams must equal n_cells when cell_stream is NULL (cell i reads stream i)");
+  TFG_CUDA(cudaSetDevice(x->device));
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (x->noise_streams_cap < n->n_streams) {
+    if (x->noise_ids) TFG_CUDA(cudaFree(x->noise_ids));
+    if (x->noise_z) TFG_CUDA(cudaFree(x->noise_z));
+    x->noise_ids = nullptr; x->noise_z = nullptr; x->noise_streams_cap = 0;
+    TFG_CUDA(cudaMalloc(&x->noise_ids, (size_t)n->n_streams * sizeof(int64_t)));
+    TFG_CUDA(cudaMalloc(&x->noise_z, 2 * (size_t)n->n_streams * sizeof(double)));
+    x->noise_streams_cap = n->n_streams;
+  }
+  if (x->noise_cells_cap < x->n_cells) {
+    if (x->noise_cell) TFG_CUDA(cudaFree(x->noise_cell));
+    x->noise_cell = nullptr; x->noise_cells_cap = 0;
+    TFG_CUDA(cudaMalloc(&x->noise_cell, (size_t)x->n_cells * sizeof(int32_t)));
+    x->noise_cells_cap = x->n_cells;
+  }
+  if (!x->noise_bad) TFG_CUDA(cudaMalloc(&x->noise_bad, sizeof(int)));
+  TFG_CUDA(cudaMemsetAsync(x->noise_bad, 0, sizeof(int), s));
+  const int64_t total = std::max<int64_t>(n->n_streams, x->n_cells);
+  noise_index_kernel<<<(unsigned)std::min<int64_t>((total + 255) / 256, 148 * 32), 256, 0, s>>>(
+      n->stream_id, n->n_streams, n->cell_stream, x->n_cells, x->noise_ids, x->noise_cell, x->noise_bad);
+  TFG_CUDA(cudaGetLastError());
+  int bad = 0;
+  TFG_CUDA(cudaMemcpyAsync(&bad, x->noise_bad, sizeof(int), cudaMemcpyDeviceToHost, s));
+  TFG_CUDA(cudaStreamSynchronize(s));
+  if (bad) {
+    std::string m = "tfg_bind_forcing_noise:";
+    if (bad & 1) m += " stream_id has negative entries;";
+    if (bad & 2) m += " cell_stream has entries outside [0, n_streams);";
+    m.pop_back();
+    return fail(m.c_str());
+  }
+  x->noise = *n;
+  x->noise.stream_id = x->noise_ids;
+  x->noise.cell_stream = x->noise_cell;
+  x->noise_c[0] = std::sqrt(1.0 - n->T_air_rho * n->T_air_rho);
+  x->noise_c[1] = std::sqrt(1.0 - n->P_rho * n->P_rho);
+  x->noise_next = -1;
+  x->have_noise = true;
+  return 0;
+}
+
+int tfg_forcing_noise_series(tfg_ctx* x, int64_t step0, int32_t n_steps, void* dT, void* fP, void* stream) {
+  if (!x || !dT || !fP) return fail("tfg_forcing_noise_series: NULL argument");
+  if (!x->have_noise) return fail("tfg_forcing_noise_series: no forcing noise bound");
+  if (n_steps <= 0) return fail("tfg_forcing_noise_series: n_steps must be > 0");
+  if (step0 < x->noise.step0) return fail("tfg_forcing_noise_series: step0 is before the bound noise's step0");
+  if (step0 + n_steps > kNoiseStepLimit) return fail("tfg_forcing_noise_series: steps must stay below 2^32");
+  TFG_CUDA(cudaSetDevice(x->device));
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int64_t S = x->noise.n_streams;
+  const unsigned grid = (unsigned)((S + 127) / 128);
+  if (x->mode == TFG_F32)
+    forcing_noise_kernel<float><<<grid, 128, 0, s>>>(noise_gen(x), x->noise_ids, S, x->noise.step0, step0, n_steps, nullptr,
+                                                     static_cast<float*>(dT), static_cast<float*>(fP), S);
+  else
+    forcing_noise_kernel<double><<<grid, 128, 0, s>>>(noise_gen(x), x->noise_ids, S, x->noise.step0, step0, n_steps,
+                                                      nullptr, static_cast<double*>(dT), static_cast<double*>(fP), S);
+  TFG_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -642,33 +858,42 @@ int tfg_run(tfg_ctx* x, const void* forcing, int64_t step0, int32_t n_steps, voi
   if (step0 + n_steps > x->n_time) return fail("tfg_run: step range exceeds the bound time table");
   if (record && (record_mask == 0 || (record_mask >> TFG_REC_COUNT) != 0)) return fail("tfg_run: bad record_mask");
   if (basin_agg && (n_basin <= 0 || !x->s.basin_id)) return fail("tfg_run: aggregates need basin_id and n_basin");
+  if (x->have_noise && step0 < x->noise.step0) return fail("tfg_run: the launch starts before the forcing noise's step0");
+  if (x->have_noise && step0 + n_steps > kNoiseStepLimit) return fail("tfg_run: forcing noise: steps must stay below 2^32");
   TFG_CUDA(cudaSetDevice(x->device));
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const bool rec = record != nullptr, agg = basin_agg != nullptr, vol = x->st.vol_P != nullptr;
   cudaError_t e = cudaSuccess;
   const size_t es = tfg_elem_size(x);
   // a launch carries at most kMaxLaunchSteps clock rows; longer runs are a sequence of launches on the same stream
-  // (bit-identical to one launch: state and snowfall window are carried through HBM either way)
-  for (int32_t t0 = 0; t0 < n_steps && e == cudaSuccess; t0 += tfg::kMaxLaunchSteps) {
-    const int32_t nt = std::min<int32_t>(tfg::kMaxLaunchSteps, n_steps - t0);
+  // (bit-identical to one launch: state and snowfall window are carried through HBM either way).  With forcing noise
+  // bound, launches are shorter where its scratch would exceed kNoiseScratchCap.
+  const int32_t per_launch = x->have_noise ? noise_launch_steps(x) : tfg::kMaxLaunchSteps;
+  for (int32_t t0 = 0; t0 < n_steps && e == cudaSuccess; t0 += per_launch) {
+    const int32_t nt = std::min<int32_t>(per_launch, n_steps - t0);
+    const int32_t want = std::min<int32_t>(per_launch, n_steps);
     const void* f = static_cast<const char*>(forcing) + (size_t)t0 * TFG_N_FORCING * (x->forcing_col ? x->n_cols : x->n_cells) * es;
     void* r = record ? static_cast<char*>(record) + (size_t)t0 * __builtin_popcountll(record_mask) * x->n_cells * es : nullptr;
     // float64 sums: 8 B per entry; exact mode: two int64 words per entry (the trailing counter stays at the end)
     void* a = basin_agg ? static_cast<char*>(basin_agg) + (size_t)t0 * n_basin * TFG_N_AGG * (x->exact_agg ? 16 : 8) : nullptr;
     long long* agg_bad = (basin_agg && x->exact_agg) ? static_cast<long long*>(basin_agg) + (size_t)n_steps * n_basin * TFG_N_AGG * 2 : nullptr;
     if (x->mode == TFG_F32) {
-      e = tfg::launch_run_f32(make_params<float>(x, f, step0 + t0, nt, r, record_mask, a, n_basin, agg_bad), rec, agg, vol, s);
+      auto p = make_params<float>(x, f, step0 + t0, nt, r, record_mask, a, n_basin, agg_bad);
+      if (x->have_noise) e = noise_pass(x, p, want, s);
+      if (e == cudaSuccess) e = tfg::launch_run_f32(p, rec, agg, vol, s);
     } else {
       auto p = make_params<double>(x, f, step0 + t0, nt, r, record_mask, a, n_basin, agg_bad);
+      if (x->have_noise) e = noise_pass(x, p, want, s);
       const bool strict = x->mode == TFG_F64_STRICT;
       // Forcing map with few columns per cell: the forcing-only part of the step is evaluated once per column and
       // timestep (column_terms_kernel, in the arithmetic of the context's mode) and the melt kernel reads one line per
       // step instead of redoing it per cell.  Same device functions either way: results do not depend on this switch
       // (test_column_terms_*).  Not for launches so small that a second kernel launch costs more than it saves
       // (per-step BMI updates of a few cells); the fast mode leaves SATTERLUND configurations to its strict step.
-      // Forcing adjustments make the forcing differ per cell, so the pass is not taken while they are bound.
+      // Forcing adjustments and forcing noise make the forcing differ per cell (or stream), so the pass is not taken
+      // while either is bound.
       const size_t need = (size_t)nt * (size_t)x->n_cols * tfg::kCtCount * sizeof(double);
-      if (x->column_terms && x->forcing_col && !x->have_fadj && !x->use_tma && (strict || !x->c.satterlund) && x->n_cols * 8 <= x->n_cells &&
+      if (e == cudaSuccess && x->column_terms && x->forcing_col && !x->have_fadj && !x->have_noise && !x->use_tma && (strict || !x->c.satterlund) && x->n_cols * 8 <= x->n_cells &&
           (int64_t)nt * x->n_cells >= 65536 && need <= (size_t(1) << 31)) {
         if (x->col_terms_bytes < need) {   // grows to the largest launch seen; a failed allocation leaves the plain path
           if (x->col_terms) cudaFree(x->col_terms);

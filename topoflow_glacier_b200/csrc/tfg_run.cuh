@@ -91,6 +91,10 @@ struct RunParams {
                                // members above, so that the kernels without aggregates keep their parameter offsets)
   const raw* fadj;             // optional [2][n_cells] T_air offset and P multiplier (tfg_bind_forcing_adjust); last, so
                                // that the kernels without adjustments keep their parameter offsets
+  // forcing noise (tfg_bind_forcing_noise), behind fadj for the same reason.  noise == nullptr: none bound
+  const raw* noise;            // [n_steps][2][n_streams]: dT and fP of this launch's steps (forcing_noise_kernel)
+  const int32_t* cell_stream;  // [n_cells] stream index of each cell, in [0, n_streams)
+  int64_t n_streams;
 };
 
 // One IEEE operation in the element type, never contracted into a neighbouring multiply-add: the forcing adjustment
@@ -216,7 +220,7 @@ struct ObjSums {
 };
 
 template <class P, bool REC, bool AGG, bool VOL, bool TMA = false, bool PRE = false, bool PAR = false, bool OBJ = false,
-          bool ADJ = false>
+          bool ADJ = false, bool NOI = false>
 __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f32 ? TFG_MIN_BLOCKS_F32 : TFG_MIN_BLOCKS)) run_kernel(const __grid_constant__ RunParams<typename P::raw> p) {
   using raw = typename P::raw;
   using R = Num<P>;
@@ -248,7 +252,16 @@ __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f3
 #pragma unroll
     for (int i = 0; i < kPCount; ++i) s.set(kSCount + i, __ldg(p.cell_par + (int64_t)i * p.n_cells + c));
   }
-  if constexpr (ADJ) { s.set(kSAdj, __ldg(p.fadj + c)); s.set(kSAdj + 1, __ldg(p.fadj + p.n_cells + c)); }
+  // NOI: forcing noise, applied after the adjustment, which these kernels always run (the identity when only noise is
+  // bound: p.fadj is warp-uniform).  The cell's stream index sits in a shared-memory column, like the adjustment.
+  static_assert(!NOI || ADJ, "forcing noise runs the forcing-adjustment kernels");
+  if constexpr (ADJ) {
+    if (!NOI || p.fadj != nullptr) { s.set(kSAdj, __ldg(p.fadj + c)); s.set(kSAdj + 1, __ldg(p.fadj + p.n_cells + c)); }
+    else { s.set(kSAdj, raw(0)); s.set(kSAdj + 1, raw(1)); }
+  }
+  __shared__ int32_t sm_noise[NOI ? kBlock : 1];
+  const unsigned noise_col = (unsigned)__cvta_generic_to_shared(&sm_noise[NOI ? threadIdx.x : 0]);
+  if constexpr (NOI) asm volatile("st.volatile.shared.s32 [%0], %1;" ::"r"(noise_col), "r"(__ldg(p.cell_stream + c)));
   s.set(kSaElev, __ldg(p.a_elev + c)); s.set(kSSinLat, __ldg(p.sin_lat + c)); s.set(kSCosLat, __ldg(p.cos_lat + c));
   s.set(kSNegTanLat, __ldg(p.neg_tan_lat + c)); s.set(kSSinEq, __ldg(p.sin_eq + c)); s.set(kSCosEq, __ldg(p.cos_eq + c));
   s.set(kSNegTanEq, __ldg(p.neg_tan_eq + c)); s.set(kSDlon, __ldg(p.dlon + c)); s.set(kSTNoon, __ldg(p.t_noon + c));
@@ -424,6 +437,13 @@ __global__ void __launch_bounds__(kBlock, P::lean ? TFG_MIN_BLOCKS_LEAN : (P::f3
     if constexpr (ADJ) {  // T_air' = T_air + offset, P' = P * multiplier: what the sanity test and both steps see
       f1 = add_once(f1, s.get(kSAdj));
       f0 = mul_once(f0, s.get(kSAdj + 1));
+    }
+    if constexpr (NOI) {  // T_air' = (T_air + offset) + dT, P' = (P * multiplier) * fP of the cell's stream at this step
+      int32_t k;
+      asm volatile("ld.volatile.shared.s32 %0, [%1];" : "=r"(k) : "r"(noise_col));
+      const raw* q = p.noise + (int64_t)t * (2 * p.n_streams) + k;
+      f1 = add_once(f1, __ldg(q));
+      f0 = mul_once(f0, __ldg(q + p.n_streams));
     }
     if constexpr (PRE && !TFG_CT_REGPF) { if (t > 0) load_line(f + (int64_t)t * (kCtCount * FN), f0, f1, f2, f3, f4, e0, e1, e2); }
     const TimeRow<raw>& row = p.rows[t];
@@ -698,6 +718,17 @@ cudaError_t launch_run_as(const RunParams<typename P::raw>& p, bool rec, bool ag
                    ((reinterpret_cast<uintptr_t>(p.forcing) & 15) == 0) &&
                    ((p.n_cells * sizeof(typename P::raw)) % 16 == 0);
   const size_t dyn = P::lean ? fm::kTabDoubles * sizeof(double) : 0;
+  if (p.noise != nullptr) {
+    // forcing noise bound: the adjustment kernels' shapes with the noise added (no column terms either)
+    if (p.obj_acc != nullptr) {
+      if (rec) run_kernel<P, true, true, true, false, false, PAR, true, true, true><<<grid, kBlock, dyn, stream>>>(p);
+      else run_kernel<P, false, true, true, false, false, PAR, true, true, true><<<grid, kBlock, dyn, stream>>>(p);
+    } else {
+      if (rec) run_kernel<P, true, true, true, false, false, PAR, false, true, true><<<grid, kBlock, dyn, stream>>>(p);
+      else run_kernel<P, false, true, true, false, false, PAR, false, true, true><<<grid, kBlock, dyn, stream>>>(p);
+    }
+    return cudaGetLastError();
+  }
   if (p.fadj != nullptr) {
     // forcing adjustments bound: the two kernel shapes of the objective, with and without it (tfg_run never binds
     // column terms then: the forcing-only terms differ per cell)
@@ -751,7 +782,8 @@ cudaError_t launch_run_as(const RunParams<typename P::raw>& p, bool rec, bool ag
 }
 
 // per-cell surface parameters bound (tfg_bind_cell_params): the PAR instantiations, chosen from the input; an objective
-// bound (p.obj_acc): the OBJ instantiations; forcing adjustments bound (p.fadj): the ADJ instantiations (launch_run_as)
+// bound (p.obj_acc): the OBJ instantiations; forcing adjustments bound (p.fadj): the ADJ instantiations; forcing noise
+// bound (p.noise): the NOI ones (launch_run_as)
 template <class P>
 cudaError_t launch_run(const RunParams<typename P::raw>& p, bool rec, bool agg, bool vol, cudaStream_t stream) {
   return p.cell_par != nullptr ? launch_run_as<P, true>(p, rec, agg, vol, stream) : launch_run_as<P, false>(p, rec, agg, vol, stream);

@@ -19,7 +19,7 @@ import torch
 
 from . import _lib
 from .config import (CELL_PARAM_KEYS, FORCING_ADJUST_IDENTITY, FORCING_ADJUST_KEYS, KERNEL_CONSTANTS, check_cell_params,
-                     check_forcing_adjust)
+                     check_forcing_adjust, check_forcing_noise)
 from .statics import cell_tables
 from .timebase import parse_start, time_tables, utc_offsets
 
@@ -60,6 +60,9 @@ class MeltEngine:
     forcing_adjust : optional mapping of ``T_air_offset`` [K] and/or ``P_multiplier`` [-] to per-cell ``[N]`` arrays or
         device tensors: every cell adds its offset to the air temperature and multiplies the precipitation rate it
         reads (its own forcing column or, with ``forcing_index``, its catchment's).  See ``set_forcing_adjust``.
+    forcing_noise : optional mapping of stochastic forcing perturbations for ensemble members: temporally correlated
+        air-temperature and log-normal precipitation noise per stream of cells, generated on the device.  See
+        ``set_forcing_noise``.
     mode : ``"f64"`` (strict), ``"f64_fast"`` or ``"f32"``
     horizon_steps : number of steps the host time tables are prepared for (extended on demand)
     """
@@ -70,7 +73,7 @@ class MeltEngine:
                  horizon_steps: int = 24 * 366, diag_integrals: bool = True, device_statics: Optional[dict] = None,
                  tma_staging: Optional[bool] = None, forcing_index=None, n_forcing_cols: Optional[int] = None,
                  column_terms: Optional[bool] = None, cell_params: Optional[Mapping] = None,
-                 forcing_adjust: Optional[Mapping] = None):
+                 forcing_adjust: Optional[Mapping] = None, forcing_noise: Optional[Mapping] = None):
         self.lib = _lib.load()
         self.device = _require_cuda(device)
         self.mode = _lib.MODE_NAMES[mode] if isinstance(mode, str) else int(mode)
@@ -132,6 +135,9 @@ class MeltEngine:
             self.forcing_adjust = None
             if forcing_adjust is not None:
                 self.set_forcing_adjust(forcing_adjust)
+            self.forcing_noise = None
+            if forcing_noise is not None:
+                self.set_forcing_noise(forcing_noise)
             self.n_cols, self.forcing_index = N, None
             if forcing_index is not None:
                 self.set_forcing_map(forcing_index, n_forcing_cols, _alloc_inputs=False)
@@ -221,6 +227,65 @@ class MeltEngine:
             # the library copies the values on the current stream and waits for its range check
             _lib.check(self.lib.tfg_bind_forcing_adjust(self.ctx, C.byref(a), self.stream_ptr), "tfg_bind_forcing_adjust")
         self.forcing_adjust = bound
+
+    def set_forcing_noise(self, noise: Optional[Mapping]) -> None:
+        """Bind stochastic forcing perturbations (``None`` unbinds them); may be called between launches.
+
+        ``noise`` maps ``T_air_sd`` (K, in [0, 5]), ``T_air_rho`` ([0, 1]), ``P_sd`` (sd of ln of the precipitation
+        factor, [0, 1.5]), ``P_rho`` ([0, 1]) and ``seed`` (an integer in [0, 2^64)); optionally ``stream``, one global
+        stream id >= 0 per cell (default: the cell index), and ``step0``, the absolute step the noise starts at
+        (default: ``step_index``, which ``load_state_dict`` restores).  Cells with the same stream id get the same noise
+        -- one stream per ensemble member perturbs a member spread over several cells coherently -- and every stream
+        is independent of the others.  At every step ``s >= step0`` cell ``i`` uses ``(T_air + T_air_offset[i]) + dT``
+        and ``(P * P_multiplier[i]) * fP`` of its stream: ``dT`` an AR(1) series of standard deviation ``T_air_sd`` and
+        lag-1 correlation ``T_air_rho``, ``fP = exp(P_sd z - P_sd^2 / 2)`` of an AR(1) series ``z`` of unit variance and
+        correlation ``P_rho``, so that ``E[fP] = 1`` (include/tfglacier.h states the definition).  The noise is a pure
+        function of (seed, stream id, step0, step): results do not depend on how a run is split into launches, on the
+        per-step path, on sharding or on a checkpoint rewind.  ``P_air``, ``Hum_sp`` and ``uz`` are not perturbed, and
+        the input block keeps what the caller set.  Values are range-checked (``ValueError``).  ``T_air_sd = P_sd = 0``
+        is not bound: the engine then runs exactly as without noise.  The noise is a binding, like
+        ``set_forcing_adjust``: ``state_dict`` does not hold it.  ``forcing_noise_series`` returns the series."""
+        if noise is None:
+            _lib.check(self.lib.tfg_bind_forcing_noise(self.ctx, None, self.stream_ptr), "tfg_bind_forcing_noise")
+            self.forcing_noise = None
+            return
+        nz = check_forcing_noise(noise)
+        stream = nz.pop("stream", None)
+        if stream is None:
+            stream = torch.arange(self.N, dtype=torch.int64, device=self.device)
+        else:
+            stream = (stream if torch.is_tensor(stream) else torch.as_tensor(np.asarray(stream, dtype=np.int64)))
+            stream = stream.to(self.device, torch.int64).reshape(-1)
+            if stream.numel() != self.N:
+                raise ValueError(f"stream: one value per cell ({self.N}) expected, got {stream.numel()}")
+        nz.setdefault("step0", self.step_index)
+        with torch.cuda.device(self.device):
+            if nz["T_air_sd"] == 0.0 and nz["P_sd"] == 0.0:
+                _lib.check(self.lib.tfg_bind_forcing_noise(self.ctx, None, self.stream_ptr), "tfg_bind_forcing_noise")
+                self.forcing_noise = None
+                return
+            ids, inv = torch.unique(stream, return_inverse=True)
+            ids, inv = ids.contiguous(), inv.to(torch.int32).contiguous()
+            b = _lib.ForcingNoise(seed=nz["seed"], step0=nz["step0"], T_air_sd=nz["T_air_sd"], T_air_rho=nz["T_air_rho"],
+                                  P_sd=nz["P_sd"], P_rho=nz["P_rho"], n_streams=ids.numel(), stream_id=ids.data_ptr(),
+                                  cell_stream=inv.data_ptr())
+            # the library copies both arrays on the current stream and waits for its range check
+            _lib.check(self.lib.tfg_bind_forcing_noise(self.ctx, C.byref(b), self.stream_ptr), "tfg_bind_forcing_noise")
+        self.forcing_noise = {**nz, "stream_id": ids, "cell_stream": inv}
+
+    def forcing_noise_series(self, step0: int, n_steps: int):
+        """``(dT, fP, stream_id)`` of the bound noise for absolute steps ``[step0, step0 + n_steps)``: ``[n_steps,
+        n_streams]`` device tensors of the engine dtype -- the values the kernel applies -- and the ``[n_streams]``
+        global ids of their columns.  Cell ``i`` reads column ``forcing_noise["cell_stream"][i]``."""
+        if self.forcing_noise is None:
+            raise RuntimeError("no forcing noise bound (set_forcing_noise)")
+        ids = self.forcing_noise["stream_id"]
+        dT = torch.empty(int(n_steps), ids.numel(), dtype=self.dtype, device=self.device)
+        fP = torch.empty_like(dT)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.tfg_forcing_noise_series(self.ctx, int(step0), int(n_steps), dT.data_ptr(), fP.data_ptr(),
+                                                         self.stream_ptr), "tfg_forcing_noise_series")
+        return dT, fP, ids
 
     # ---- objective: scores of every cell against observations, accumulated inside the melt kernel ----------------
     def set_objective(self, quantity: Optional[str], obs=None, obs_step0: int = 0, obs_index=None) -> None:

@@ -212,11 +212,14 @@ class ShardedMeltEngine:
     ``n_total``.  ``basin_id`` / ``tz_idx`` / ``forcing_index`` are global arrays (or callables ``(lo, hi)``); so is
     ``cell_params``: a mapping of global per-cell parameter arrays (``MeltEngine(cell_params=...)``), sliced here, or a
     callable ``(lo, hi) -> mapping`` of the shard's arrays; ``forcing_adjust`` likewise (``MeltEngine(forcing_adjust=...)``).
+    ``forcing_noise`` (``MeltEngine(forcing_noise=...)``) takes a global per-cell ``stream``, sliced here; without one
+    every cell is its own stream with its GLOBAL cell index as id, so that the ranks together equal one engine.
     Attribute access falls through to the local ``MeltEngine`` (``state``, ``row``, ``step_index`` ...).
     """
 
     def __init__(self, cells, consts, start_time, *, n_total: Optional[int] = None, basin_id=None, n_basin: int = 0,
-                 tz_idx=None, forcing_index=None, cell_params=None, forcing_adjust=None, group=None, exact: bool = True,
+                 tz_idx=None, forcing_index=None, cell_params=None, forcing_adjust=None, forcing_noise=None, group=None,
+                 exact: bool = True,
                  device: Optional[int] = None, **kw):
         import os
 
@@ -249,12 +252,16 @@ class ShardedMeltEngine:
         if forcing_adjust is not None:
             forcing_adjust = (forcing_adjust(lo, hi) if callable(forcing_adjust)
                               else {k: v[lo:hi] for k, v in forcing_adjust.items()})
+        if forcing_noise is not None:
+            forcing_noise = dict(forcing_noise)
+            st = forcing_noise.get("stream")
+            forcing_noise["stream"] = np.arange(lo, hi, dtype=np.int64) if st is None else st[lo:hi]
         dev_tables = "a_elev" in local
         self.exact = bool(exact)
         self.engine = MeltEngine(None if dev_tables else local, consts, start_time, basin_id=part(basin_id),
                                  n_basin=n_basin, tz_idx=part(tz_idx), forcing_index=part(forcing_index), device=device,
                                  device_statics=local if dev_tables else None, cell_params=cell_params,
-                                 forcing_adjust=forcing_adjust, **kw)
+                                 forcing_adjust=forcing_adjust, forcing_noise=forcing_noise, **kw)
         self._aggs: dict = {}
 
     def __getattr__(self, name):
